@@ -1,7 +1,7 @@
 """
 bench.py - headline benchmark of the DCSCN hot path (BASELINE.json: "output Mpixels/sec DCSCN L12 x2").
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
   torchrun --nnodes=1 --nproc-per-node N ... bench.py --gpus N --steps K --warmup W
 
 Headline: a "step" is one forward pass of DCSCN L12 F196->48 x2 over one batch of 256 synthetic 48x48 Y tiles
@@ -294,6 +294,7 @@ def umma_isolated(device):
 
 
 def headline(job, args):
+    import numpy as np
     import torch
     from helper import engine as E
     rank, world = job.rank, job.world
@@ -325,6 +326,10 @@ def headline(job, args):
     ms = job.max_over_ranks(ev0.elapsed_time(ev1))
     launches = eng.launch_count - launches0
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        # y of the last timed step, before the strict pass below overwrites it with another promotion setting
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "y.npy"), y.cpu().numpy())
     out_px_step = BATCH * (SCALE * TILE) ** 2
     value = world * out_px_step * args.steps / (ms / 1e3) / 1e6
 
@@ -612,7 +617,14 @@ def main():
     ap.add_argument("--no-sub", action="store_false", dest="sub", help="headline only (skip ensemble8 / train / ds / latency)")
     ap.add_argument("--workload", default="infer", choices=["infer", "train", "ds", "ensemble", "latency"],
                     help="infer = headline line with all sub-records; the others print one sub-record alone")
+    ap.add_argument("--dump-outputs", default=None, dest="dump_outputs", metavar="DIR",
+                    help="write the headline's output of its last timed step (rank 0) as DIR/y.npy, float32 "
+                         "[256, 96, 96, 1]; the inputs are seeded, so two builds can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload != "infer"):
+        ap.error("--dump-outputs writes the headline's output: it needs --impl ours --workload infer")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
