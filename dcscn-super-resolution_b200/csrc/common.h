@@ -74,20 +74,16 @@ struct ConvTCParams {
   ConvGeom g;
   int ksz;               // 1 or 3
   int cin_pad;           // padded input channels of the source slot (multiple of 16)
-  int chunks;            // ceil(cin_pad / KC)
+  int chunks;            // ceil(cin_pad / 64)
   int n_tiles;           // column tiles (N > 256 is split)
   int n_pad;             // columns per tile, multiple of 16, <= 256
   int seg_chunks;        // pipeline stages per accumulation segment (fp32 promotion period)
-  int cluster_size;      // CTAs per cluster sharing (multicasting) the weight tiles: 1, 2 or 4
-  const __half* wpack;   // packed weights [n_tile][tap][chunk][plane][n_pad x KC] (pre-swizzled)
-  // streaming kernel (conv_tc_halo2.cuh): weight-stage table of one (pixel tile, column tile) item, see kH2* there
-  const uint32_t* h2_stages;
-  int h2_nstages;
+  // streaming kernel (conv_tc_halo2.cuh)
+  int h2_nstages;        // weight stages of one (pixel tile, column tile) item: 9 per channel chunk
   int h2_nseg;           // fp32-promotion segments per item
   int h2_resident;       // all stages fit in shared memory: loaded once per CTA
   int pair_stream;       // conv_tc_pair_kernel: streaming split-accumulator mode (1x1 layers)
   unsigned long long* dbg;   // diagnostic builds (-DDCSCN_H2_DEBUG): per-cluster wait counters, else null
-  int h2_nreg;           // leading chunks with one tap per stage (issued by the compile-time-structured loop)
   EpiParams epi;
 };
 

@@ -1,13 +1,13 @@
-// Implicit-GEMM convolution on tcgen05 tensor cores (sm_100a).
+// Implicit-GEMM convolution on tcgen05 tensor cores (sm_100a): what the CTA-pair kernel (conv_tc_pair.cuh), the
+// streaming 3x3 kernel (conv_tc_halo2.cuh) and the UMMA probe (umma_probe.cuh) share.
 //
 // Replaces  tf.nn.conv2d(SAME, stride 1, NHWC, HWIO) + bias + PReLU  of the reference
 // (helper/tf_graph.py:104-153 conv2d / build_conv; :238-249 build_pixel_shuffler_layer).
 //
-// GEMM view:  D[M = 128 pixels (TH x TW patch), N = cout (padded to 16)]
-//             = sum over taps (ky,kx) and input-channel chunks of  A_tap[128 x KC] * W_tap[KC x N]
-//   * A tiles are fetched by TMA (4-D tiled tensor map over the NHWC fp16 plane, box {KC, TW, TH, 1});
-//     the box origin is shifted by the tap offset and TMA zero-fills out-of-image pixels, which IS
-//     TF's SAME padding - no halo handling in the kernel.
+// GEMM view:  D[M = 128 pixels (TH x TW patch) per CTA, N = cout (padded to 16)]
+//             = sum over taps (ky,kx) and 64-channel chunks of  A_tap[128 x 64] * W_tap[64 x N]
+//   * A tiles are fetched by TMA (4-D tiled tensor map over the NHWC fp16 plane, SWIZZLE_128B); TMA zero-fills
+//     out-of-image pixels, which IS TF's SAME padding - no bounds handling in the kernels.
 //   * fp32-equivalent precision from fp16 tensor cores:  a = a_hi + a_lo,  w*2^s = w_hi + w_lo
 //     (each 11-bit significands), D += a_hi*w_hi + a_lo*w_hi + a_hi*w_lo   (3 x kind::f16 UMMA,
 //     fp32 accumulation in TMEM).  NPLANES == 1 is the single-pass fp16 "fast" mode.
@@ -16,10 +16,6 @@
 //     333 UMMAs of CNN2).  K is therefore cut into short segments (`seg_chunks` pipeline stages): each segment
 //     accumulates in TMEM from zero, and the epilogue warps add the segment sums into fp32 registers with
 //     round-to-nearest ("promotion"), double-buffered against the next segment's UMMAs.
-//   * Weight tiles are the dominant L2->SM traffic (every 128-pixel tile streams the whole layer's weights).  CTAs
-//     are launched in clusters of `cs` (1, 2 or 4) that walk pixel tiles in lockstep; each CTA fetches 1/cs of
-//     every weight tile and multicasts it to the whole cluster (cp.async.bulk ... .multicast::cluster), and every
-//     CTA's MMA warp releases a pipeline stage in all cluster members (tcgen05.commit ... .multicast::cluster).
 //   * Warp roles: warp 0 = TMA producer, warp 1 = MMA issuer (+TMEM alloc), warps 4..11 = epilogue (registers re-balanced with setmaxnreg)
 //     (TMEM -> registers, running fp32 sums, then bias/PReLU/split -> global), persistent CTAs striding
 //     over (pixel-tile, column-tile) work items.
@@ -49,19 +45,9 @@ struct TcSmem {
   static constexpr uint64_t kLayout = (KC == 64) ? 2ull : 4ull;  // UMMA LayoutType: SW128 = 2, SW64 = 4
 };
 
-// Shared-memory matrix descriptor for a K-major swizzled operand tile (cute::UMMA::SmemDescriptor).
-template <int KC>
-__device__ __forceinline__ uint64_t make_smem_desc(uint32_t saddr) {
-  uint64_t d = 0;
-  d |= (uint64_t)((saddr & 0x3FFFFu) >> 4);              // start address  [0,14)
-  d |= (uint64_t)1 << 16;                                // leading byte offset (unused for swizzled K-major)
-  d |= (uint64_t)(TcSmem<KC>::kSbo >> 4) << 32;          // stride byte offset [32,46)
-  d |= (uint64_t)1 << 46;                                // descriptor version (Blackwell)
-  d |= TcSmem<KC>::kLayout << 61;                        // swizzle mode
-  return d;
-}
-
-// Split form for the issue loop: the upper word is constant, the lower word is (address >> 4) | LBO.
+// Shared-memory matrix descriptor for a K-major swizzled operand tile (cute::UMMA::SmemDescriptor), split for the issue
+// loops: the upper word is constant (SBO [32,46), descriptor version bit 46, swizzle mode [61,64)), the lower word is
+// (start address >> 4) | LBO (unused for swizzled K-major).
 template <int KC>
 __device__ __forceinline__ uint32_t desc_lo_t(uint32_t saddr) {
   return ((saddr & 0x3FFFFu) >> 4) | (1u << 16);
@@ -75,283 +61,6 @@ __device__ __forceinline__ uint64_t make_desc64_t(uint32_t lo) {
 // kind::f16 instruction descriptor: fp16 x fp16 -> fp32, A and B K-major, M = 128, N = n_pad.
 __device__ __forceinline__ uint32_t make_idesc_f16(int n_pad) {
   return (1u << 4) | ((uint32_t)(n_pad >> 3) << 17) | ((uint32_t)(kTileM >> 4) << 24);
-}
-
-__host__ __device__ inline size_t tc_stage_bytes(int KC, int nplanes, int n_pad) {
-  return (size_t)nplanes * ((size_t)kTileM * KC * 2 + (size_t)n_pad * KC * 2);
-}
-
-template <int KC, int NPLANES>
-__global__ void __launch_bounds__(kTcThreads, 1)
-conv_tc_kernel(const __grid_constant__ CUtensorMap tm_hi, const __grid_constant__ CUtensorMap tm_lo,
-               const ConvTCParams p, const int num_stages) {
-  extern __shared__ __align__(1024) uint8_t smem_raw[];
-  // carve: [stages x (A_hi, A_lo, B_hi, B_lo)] then barriers
-  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
-  constexpr int A_BYTES = TcSmem<KC>::kABytes;
-  const int B_BYTES = p.n_pad * KC * 2;
-  const int STAGE_BYTES = NPLANES * (A_BYTES + B_BYTES);
-  uint64_t* full_bar = reinterpret_cast<uint64_t*>(smem + (size_t)num_stages * STAGE_BYTES);
-  uint64_t* empty_bar = full_bar + kMaxStages;
-  uint64_t* acc_full = empty_bar + kMaxStages;
-  uint64_t* acc_empty = acc_full + kAccStages;
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(acc_empty + kAccStages);
-  float* s_rdot = reinterpret_cast<float*>(tmem_slot + 4);   // 16-byte aligned (barriers start 1024-aligned)
-
-  const int warp = threadIdx.x >> 5;
-  const int lane = threadIdx.x & 31;
-  const int cs = p.cluster_size;
-  const uint32_t rank = cs > 1 ? ptx::cluster_ctarank() : 0u;
-  const uint16_t cta_mask = (uint16_t)((1u << cs) - 1u);
-
-  if (threadIdx.x == 0) {
-    for (int s = 0; s < num_stages; ++s) {
-      ptx::mbar_init(&full_bar[s], 1);
-      ptx::mbar_init(&empty_bar[s], cs);        // one tcgen05.commit arrival from every CTA of the cluster
-    }
-    for (int s = 0; s < kAccStages; ++s) {
-      ptx::mbar_init(&acc_full[s], 1);
-      ptx::mbar_init(&acc_empty[s], kEpiWarps);  // one arrive per epilogue warp
-    }
-    ptx::fence_barrier_init();
-    ptx::fence_proxy_async();
-  }
-  if (warp == 1) {
-    ptx::tmem_alloc(tmem_slot, kAccStages * kAccStride);
-    ptx::tmem_relinquish();
-  }
-  if (p.epi.mode == EPI_D2S_RDOT)
-    for (int i = threadIdx.x; i < p.epi.rdot_taps * p.epi.d2s_cout; i += blockDim.x) s_rdot[i] = p.epi.rdot_w[i];
-  ptx::tc_fence_before();
-  __syncthreads();
-  if (cs > 1) ptx::cluster_sync();               // peers' barriers are initialised before anything targets them
-  ptx::tc_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
-
-  const ConvGeom& g = p.g;
-  const int tiles_per_img = g.tiles_x * g.tiles_y;
-  const int num_tiles = g.n_img * tiles_per_img;
-  const int groups = (num_tiles + cs - 1) / cs;  // cs pixel tiles are processed by one cluster iteration
-  const int num_items = groups * p.n_tiles;
-  const int cluster_id = blockIdx.x / cs;
-  const int num_clusters = gridDim.x / cs;
-  const int taps = p.ksz * p.ksz;
-  const int half = p.ksz >> 1;
-  const int total_chunks = taps * p.chunks;
-
-  if (warp < kEpiWarp0) {
-    ptx::setmaxnreg_dec<kRegsIssue>();
-    if (warp == 0) {
-      // ============================== TMA producer ==============================
-      if (lane == 0) {
-        ptx::prefetch_tensormap(&tm_hi);
-        if (NPLANES == 2) ptx::prefetch_tensormap(&tm_lo);
-        const int slice_rows = p.n_pad / cs;                       // this CTA's share of every weight tile
-        const uint32_t slice_bytes = (uint32_t)(slice_rows * KC * 2);
-        const uint32_t slice_off = rank * slice_bytes;
-        int stage = 0;
-        uint32_t phase = 0;
-        for (int item = cluster_id; item < num_items; item += num_clusters) {
-          const int n_tile = item % p.n_tiles;
-          int tile = (item / p.n_tiles) * cs + (int)rank;
-          if (tile >= num_tiles) tile = num_tiles - 1;             // lockstep filler (stores are masked)
-          const int img = tile / tiles_per_img;
-          const int t2 = tile - img * tiles_per_img;
-          const int ty = t2 / g.tiles_x, tx = t2 - ty * g.tiles_x;
-          const uint8_t* wsrc = reinterpret_cast<const uint8_t*>(p.wpack) +
-                                (size_t)n_tile * total_chunks * (size_t)(NPLANES * B_BYTES);
-          for (int tap = 0; tap < taps; ++tap) {
-            const int dy = tap / p.ksz - half, dx = tap % p.ksz - half;
-            for (int ch = 0; ch < p.chunks; ++ch) {
-              ptx::mbar_wait(&empty_bar[stage], phase ^ 1);
-              uint8_t* st = smem + (size_t)stage * STAGE_BYTES;
-              ptx::mbar_arrive_expect_tx(&full_bar[stage], (uint32_t)STAGE_BYTES);
-              ptx::tma_load_4d(st, &tm_hi, &full_bar[stage], ch * KC, tx * g.TW + dx, ty * g.TH + dy, img);
-              if (NPLANES == 2)
-                ptx::tma_load_4d(st + A_BYTES, &tm_lo, &full_bar[stage], ch * KC, tx * g.TW + dx, ty * g.TH + dy, img);
-              const uint8_t* wtile = wsrc + (size_t)(tap * p.chunks + ch) * (NPLANES * B_BYTES);
-              uint8_t* bdst = st + NPLANES * A_BYTES;
-              if (cs == 1) {
-                ptx::bulk_load(bdst, wtile, (uint32_t)(NPLANES * B_BYTES), &full_bar[stage]);
-              } else {
-#pragma unroll
-                for (int pl = 0; pl < NPLANES; ++pl)
-                  ptx::bulk_load_multicast(bdst + pl * B_BYTES + slice_off, wtile + (size_t)pl * B_BYTES + slice_off,
-                                           slice_bytes, &full_bar[stage], cta_mask);
-              }
-              if (++stage == num_stages) { stage = 0; phase ^= 1; }
-            }
-          }
-        }
-      }
-    } else if (warp == 1) {
-      // ============================== MMA issuer ================================
-      const uint32_t idesc = make_idesc_f16(p.n_pad);
-      const uint32_t smem_base_u32 = ptx::smem_u32(smem);
-      int stage = 0;
-      uint32_t phase = 0;
-      uint32_t seg_count = 0;
-      for (int item = cluster_id; item < num_items; item += num_clusters) {
-        for (int c0 = 0; c0 < total_chunks; c0 += p.seg_chunks) {
-          const int acc = seg_count & 1;
-          ptx::mbar_wait(&acc_empty[acc], ((seg_count >> 1) & 1) ^ 1);
-          ptx::tc_fence_after();
-          const uint32_t tmem_d = tmem_base + (uint32_t)(acc * kAccStride);
-          uint32_t accumulate = 0;  // every segment starts from zero
-          const int c1 = (c0 + p.seg_chunks < total_chunks) ? c0 + p.seg_chunks : total_chunks;
-          // Pass A: as the stages of this segment land, issue the small correction products (a_lo*w_hi, a_hi*w_lo).
-          // Pass B: the dominant a_hi*w_hi products, releasing each stage.  The accumulator only becomes large in
-          // pass B, so only those UMMAs contribute truncation error: 3x fewer "effective" steps per segment.
-          // Warp-uniform descriptor arithmetic; only the UMMA / commit instructions are single-lane (elect.sync), which
-          // keeps the issue loop on the uniform datapath.
-          int st = stage;
-          uint32_t ph = phase;
-          for (int c = c0; c < c1; ++c) {
-            const int ch = c % p.chunks;
-            ptx::mbar_wait(&full_bar[st], ph);
-            ptx::tc_fence_after();
-            if (NPLANES == 2) {
-              const uint32_t st_addr = smem_base_u32 + (uint32_t)st * (uint32_t)STAGE_BYTES;
-              const uint32_t la_hi = desc_lo_t<KC>(st_addr);
-              const uint32_t la_lo = desc_lo_t<KC>(st_addr + A_BYTES);
-              const uint32_t lb_hi = desc_lo_t<KC>(st_addr + NPLANES * A_BYTES);
-              const uint32_t lb_lo = desc_lo_t<KC>(st_addr + NPLANES * A_BYTES + B_BYTES);
-              int ksteps = (p.cin_pad - ch * KC);
-              ksteps = (ksteps > KC ? KC : ksteps) >> 4;
-              if (ptx::elect_one()) {
-#pragma unroll 1
-                for (int ks = 0; ks < ksteps; ++ks) {
-                  const uint32_t kadd = (uint32_t)ks * 2u;  // 32 bytes (16 fp16 along K) in 16-byte descriptor units
-                  ptx::mma_f16_ss(tmem_d, make_desc64_t<KC>(la_lo + kadd), make_desc64_t<KC>(lb_hi + kadd), idesc, accumulate);
-                  ptx::mma_f16_ss(tmem_d, make_desc64_t<KC>(la_hi + kadd), make_desc64_t<KC>(lb_lo + kadd), idesc, 1);
-                  accumulate = 1;
-                }
-              }
-              accumulate = 1;
-              __syncwarp();
-            }
-            if (++st == num_stages) { st = 0; ph ^= 1; }
-          }
-          st = stage;
-          for (int c = c0; c < c1; ++c) {
-            const int ch = c % p.chunks;
-            const uint32_t st_addr = smem_base_u32 + (uint32_t)st * (uint32_t)STAGE_BYTES;
-            const uint32_t la_hi = desc_lo_t<KC>(st_addr);
-            const uint32_t lb_hi = desc_lo_t<KC>(st_addr + NPLANES * A_BYTES);
-            int ksteps = (p.cin_pad - ch * KC);
-            ksteps = (ksteps > KC ? KC : ksteps) >> 4;
-            if (ptx::elect_one()) {
-#pragma unroll 1
-              for (int ks = 0; ks < ksteps; ++ks) {
-                const uint32_t kadd = (uint32_t)ks * 2u;
-                ptx::mma_f16_ss(tmem_d, make_desc64_t<KC>(la_hi + kadd), make_desc64_t<KC>(lb_hi + kadd), idesc, accumulate);
-                accumulate = 1;
-              }
-              if (cs == 1) ptx::mma_commit(&empty_bar[st]); else ptx::mma_commit_multicast(&empty_bar[st], cta_mask);  // frees this smem stage once the UMMAs have read it
-            }
-            accumulate = 1;
-            __syncwarp();
-            if (++st == num_stages) st = 0;
-          }
-          stage = st;
-          phase = ph;
-          if (ptx::elect_one()) ptx::mma_commit(&acc_full[acc]);  // segment complete -> epilogue promotes it
-          __syncwarp();
-          ++seg_count;
-        }
-      }
-    }
-  } else {
-    ptx::setmaxnreg_inc<kRegsEpilogue>();
-    // ============================== epilogue ==================================
-    const int ew = warp - kEpiWarp0;
-    const int quad = warp & 3;               // TMEM lane quadrant this warp may access
-    const int grp = ew >> 2;                 // which group of columns this warp owns
-    const int row = quad * 32 + lane;        // pixel index inside the TH x TW patch
-    const int py = row / g.TW, px = row - py * g.TW;
-    const int n_total = p.n_tiles * p.n_pad;
-    const int nch = p.n_pad >> 4;
-    const int per = (nch + kColSplit - 1) / kColSplit;
-    const int first_chunk = grp * per;
-    const int my_chunks = (nch - first_chunk) < per ? ((nch - first_chunk) > 0 ? nch - first_chunk : 0) : per;
-    const int col_base = first_chunk * 16;
-    const int nseg = (total_chunks + p.seg_chunks - 1) / p.seg_chunks;
-    const uint32_t taddr0 = tmem_base + ((uint32_t)(quad * 32) << 16) + (uint32_t)col_base;
-    uint32_t seg_count = 0;
-    for (int item = cluster_id; item < num_items; item += num_clusters) {
-      const int n_tile = item % p.n_tiles;
-      const int tile = (item / p.n_tiles) * cs + (int)rank;
-      const bool real = tile < num_tiles;
-      const int img = tile / tiles_per_img;
-      const int t2 = tile - img * tiles_per_img;
-      const int ty = t2 / g.tiles_x, tx = t2 - ty * g.tiles_x;
-      const int y = ty * g.TH + py, x = tx * g.TW + px;
-      const bool valid = real && (y < g.H) && (x < g.W);
-
-      float sum[kMaxColChunks][16];
-#pragma unroll
-      for (int j = 0; j < kMaxColChunks; ++j)
-#pragma unroll
-        for (int i = 0; i < 16; ++i) sum[j][i] = 0.f;
-      for (int s = 0; s < nseg; ++s) {
-        const int acc = seg_count & 1;
-        ptx::mbar_wait(&acc_full[acc], (seg_count >> 1) & 1);
-        ptx::tc_fence_after();
-        const uint32_t taddr = taddr0 + (uint32_t)(acc * kAccStride);
-        // fp32 round-to-nearest promotion of the segment: wide TMEM loads (64 / 32 columns per instruction); columns
-        // past this thread's share may be read (they stay inside the accumulator stage) but are never stored.
-#pragma unroll
-        for (int j = 0; j < kMaxColChunks; j += 4) {
-          if (j < my_chunks) {
-            if (my_chunks - j > 2) {
-              float v[64];
-              ptx::tmem_ld64(taddr + j * 16, v);
-#pragma unroll
-              for (int i = 0; i < 64; ++i) sum[j + (i >> 4)][i & 15] += v[i];
-            } else {
-              float v[32];
-              ptx::tmem_ld32(taddr + j * 16, v);
-#pragma unroll
-              for (int i = 0; i < 32; ++i) sum[j + (i >> 4)][i & 15] += v[i];
-            }
-          }
-        }
-        ptx::tc_fence_before();
-        __syncwarp();
-        if (lane == 0) ptx::mbar_arrive(&acc_empty[acc]);
-        ++seg_count;
-      }
-      if (p.epi.mode == EPI_D2S_RDOT) {
-        // this thread owns whole sub-pixel channel groups (host guarantees (columns per thread) % d2s_cout == 0)
-        float v[9];
-#pragma unroll
-        for (int t = 0; t < 9; ++t) v[t] = 0.f;
-#pragma unroll
-        for (int j = 0; j < kMaxColChunks; ++j) {
-          if (j < my_chunks) {
-            const int cg = n_tile * p.n_pad + col_base + j * 16;
-            if (cg < p.epi.n_valid) {
-              const int ij = cg / p.epi.d2s_cout, c = cg - ij * p.epi.d2s_cout;
-              rdot_accumulate16(p.epi, s_rdot, cg, c, sum[j], v);
-              if (c + 16 == p.epi.d2s_cout && valid) rdot_flush(p.epi, g, img, y, x, ij, v);
-            }
-          }
-        }
-      } else if (valid) {
-#pragma unroll
-        for (int j = 0; j < kMaxColChunks; ++j)
-          if (j < my_chunks) epilogue_store16(p.epi, g, n_total, img, y, x, n_tile * p.n_pad + col_base + j * 16, sum[j]);
-      }
-    }
-  }
-
-  ptx::tc_fence_before();
-  __syncthreads();
-  if (cs > 1) ptx::cluster_sync();  // nobody exits while a peer may still signal its barriers
-  if (warp == 1) {
-    ptx::tc_fence_after();
-    ptx::tmem_dealloc(tmem_base, kAccStages * kAccStride);
-  }
 }
 
 }  // namespace dcscn

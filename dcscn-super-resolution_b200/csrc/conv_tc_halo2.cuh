@@ -1,44 +1,50 @@
-// Streaming variant of the single-box halo kernel (conv_tc_halo1.cuh): same operands, same TMA boxes, same three
-// kind::f16 products per algorithmic MAC - but a weight stage is RELEASED as soon as its three products are issued.
+// Streaming halo kernel of the 3x3 layers: CTA-pair tcgen05 convolution (see conv_tc_pair.cuh) whose A operand is read
+// once per channel chunk for all nine taps, and whose weight stages are released as soon as their products are issued.
 //
-// Why (profiles/r1d_conv_tc_ncu_summary.csv): conv_tc_halo1 keeps all weight stages of an fp32-promotion segment
-// resident for two passes (small correction products first, dominant a_hi*w_hi last, so that only 1/3 of the UMMAs
-// see a large accumulator - the tensor core truncates its fp32 accumulate on every UMMA).  With 22 KB stages only two
-// of the five ring slots were ever free for prefetch, and every layer ran at ~4.5 TB/s of TMA traffic into shared
-// memory whatever its shape: latency-bound on the weight ring, tensor pipe 31-50 % active.
+// A operand: the pixel patch is 16 rows x 8 columns.  Per 64-channel chunk ONE {64, 10, 18, 1} TMA box (the patch and
+// its one-pixel halo, 180 smem rows of 128 B) serves all nine taps.  The smem rows are (hy * 10 + hx); tap (dy, dx)
+// starts (dy * 10 + dx) rows into the box, and the 16 eight-row groups of the UMMA A operand are 10 rows (1280 B) apart,
+// so operand rows are NOT aligned to the 1024-byte swizzle atom.  This relies on the tensor core applying the 128B-swizzle
+// XOR on absolute shared-memory address bits [7,10), like TMA does when writing - measured on B200: correct with the
+// descriptor base-offset field left 0, wrong with it set to the operand's offset inside the atom.
 //
-// Here the two kinds of products go to DIFFERENT TMEM accumulators, so the order of issue inside a stage no longer
-// matters for accuracy and nothing has to be held:
-//   * the K loop of a tile is cut into segments s = 0..nseg-1 as before; accumulation "slot" j = 0..nseg receives the
-//     correction products (a_lo*w_hi, a_hi*w_lo) of segment j-1 FIRST (while it is still small) and the dominant
-//     products of segment j afterwards;  slot j is complete at the end of segment j and the epilogue warps add it into
-//     their fp32 registers with round-to-nearest ("promotion").  One more drain per tile than halo1 (nseg + 1).
-//   * slots rotate over THREE TMEM buffers of n_pad columns: during segment s buffer (s % 3) takes dominant products,
-//     ((s + 1) % 3) corrections, ((s + 2) % 3) is being drained.  3 * n_pad <= 512 columns -> n_pad <= 160; wider
-//     layers are split into column tiles by the engine (choose_tiling).
+// B operand: one weight stage = one [n_pad/2 rows x 128 bytes] (x planes) operand tile per CTA = the four 16-channel K
+// slices of one tap of one chunk.  Stages are ordered [chunk][dx][dy] (host: pair_image in engine.cu); a last chunk with
+// 16, 32 or 48 valid channels (cin_pad % 64) issues only its first 1, 2 or 3 slices.
+//
+// Accumulation: three kind::f16 products per algorithmic MAC (conv_tc.cuh).  The tensor core truncates its fp32
+// accumulate on every UMMA, so the K loop of a tile is cut into fp32-promotion segments, and the two kinds of products go
+// to DIFFERENT TMEM accumulators - the order of issue inside a stage does not matter for accuracy and no stage is held
+// for a second pass (profiles/r1d_conv_tc_ncu_summary.csv: round 1's two-pass 3x3 kernel, which kept a segment's stages
+// resident until its dominant pass, left two of five 22 KB ring slots free for prefetch and ran every layer at
+// ~4.5 TB/s of TMA traffic into shared memory, tensor pipe 31-50 % active):
+//   * segments s = 0..nseg-1 end at (chunk, dx) boundaries; accumulation "slot" j = 0..nseg receives the correction
+//     products (a_lo*w_hi, a_hi*w_lo) of segment j-1 FIRST (while it is still small) and the dominant products of
+//     segment j afterwards;  slot j is complete at the end of segment j and the epilogue warps add it into their fp32
+//     registers with round-to-nearest ("promotion").  nseg + 1 drains per tile.
+//   * slots rotate over the TMEM buffers of n_pad columns: with three, during segment s buffer (s % 3) takes dominant
+//     products, ((s + 1) % 3) corrections, ((s + 2) % 3) is being drained.  3 * n_pad <= 512 columns -> n_pad <= 160;
+//     wider layers are split into column tiles by the engine (choose_tiling) or run on two buffers (option "wide_tiles").
 //   * every stage of the weight ring and every A slot is released by the tcgen05.commit that follows its last UMMA,
-//     so the whole ring (up to 24 stages) is prefetch depth.
+//     so the whole ring (up to 32 stages) is prefetch depth.
 #pragma once
-#include "conv_tc_halo1.cuh"
+#include "conv_tc_pair.cuh"
 
 namespace dcscn {
 
+constexpr int kHaloTW = 8, kHaloTH = 16;                          // pixel patch of one CTA
+constexpr int kHalo1W = kHaloTW + 2;                              // 10 columns
+constexpr int kHalo1Rows = (kHaloTH + 2) * kHalo1W;               // 180 rows
+constexpr int kHalo1PlaneBytes = ((kHalo1Rows * 128 + 1023) / 1024) * 1024;  // 23552, keeps planes 1024-aligned
+
+__host__ __device__ inline size_t tc_halo1_a_slot_bytes(int nplanes) { return (size_t)nplanes * kHalo1PlaneBytes; }
+__host__ __device__ inline size_t tc_halo_b_stage_bytes(int nplanes, int n_pad) {
+  return (size_t)nplanes * (size_t)(n_pad / 2) * 128;
+}
+
 constexpr int kH2MaxStages = 32;
 constexpr int kH2MaxAcc = 4;
-constexpr int kH2BarBytes = 2048;        // mbarriers (4 x 32 + 2 x 4) + TMEM slot + the stage table
-constexpr int kH2MaxTable = 64;          // weight stages of one item (9 taps x up to 4 channel chunks, packed tails fewer)
-constexpr int kH2TableOff = 1280;        // byte offset of the stage table inside the barrier block
-
-// One weight stage = one [n_pad/2 rows x 128 bytes] (x planes) operand tile per CTA = four 16-channel K slices.
-// A full 64-channel chunk uses one stage per filter tap (4 slices of that tap).  The LAST chunk of a layer often holds
-// only 16 or 32 valid channels (cin_pad % 64): its stages pack the slices of 4 (or 2) consecutive taps, so no zero
-// columns are streamed from L2 - 9 tail stages shrink to 3 (or 5).  Stage word (host: build_h2_stages in engine.cu):
-//   bits 0-7 channel chunk | 8-11 taps in the stage | 12-15 first tap (dx * 3 + dy) | 16-19 16-channel slices per tap |
-//   bit 20 first stage of its chunk (wait for the A box) | bit 21 last stage of its chunk (release the A box) |
-//   bit 22 last stage of an fp32-promotion segment.
-// A second word per stage carries, 8 bits per tap, the tap's first row inside the halo box (dy * 10 + dx): the issuing
-// thread does no division.
-constexpr uint32_t kH2ChunkFirst = 1u << 20, kH2ChunkLast = 1u << 21, kH2SegEnd = 1u << 22;
+constexpr int kH2BarBytes = 2048;        // mbarriers (4 x 32 + 2 x 4) + TMEM slot, with room to spare: the engine sizes the rings from it
 
 __host__ __device__ inline size_t tc_halo2_misc_bytes() { return 1024 + kH2BarBytes + kRdotSmemBytes; }
 
@@ -55,8 +61,7 @@ __host__ __device__ inline size_t tc_halo2_misc_bytes() { return 1024 + kH2BarBy
 template <int NPLANES>
 __global__ void __launch_bounds__(kTcThreads, 1)
 conv_tc_halo2_kernel(const __grid_constant__ CUtensorMap tm_hi, const __grid_constant__ CUtensorMap tm_lo,
-                     const __grid_constant__ CUtensorMap tm_w, const ConvTCParams p, const int num_a, const int num_b,
-                     const int wide_w) {
+                     const __grid_constant__ CUtensorMap tm_w, const ConvTCParams p, const int num_a, const int num_b) {
   constexpr int KC = 64;
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
@@ -74,7 +79,6 @@ conv_tc_halo2_kernel(const __grid_constant__ CUtensorMap tm_hi, const __grid_con
   uint64_t* acc_full = b_empty + kH2MaxStages;
   uint64_t* acc_empty = acc_full + kH2MaxAcc;
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(acc_empty + kH2MaxAcc);
-  uint32_t* s_tab = reinterpret_cast<uint32_t*>(reinterpret_cast<uint8_t*>(a_full) + kH2TableOff);
   float* s_rdot = reinterpret_cast<float*>(reinterpret_cast<uint8_t*>(a_full) + kH2BarBytes);
 
   const int warp = threadIdx.x >> 5;
@@ -108,8 +112,7 @@ conv_tc_halo2_kernel(const __grid_constant__ CUtensorMap tm_hi, const __grid_con
   }
   if (p.epi.mode == EPI_D2S_RDOT)
     for (int i = threadIdx.x; i < p.epi.rdot_taps * p.epi.d2s_cout; i += blockDim.x) s_rdot[i] = p.epi.rdot_w[i];
-  const int nst = p.h2_nstages;
-  for (int i = threadIdx.x; i < 2 * nst; i += blockDim.x) s_tab[i] = p.h2_stages[i];
+  const int nst = p.h2_nstages;                       // weight stages of one item: 9 per channel chunk
   ptx::tc_fence_before();
   __syncthreads();
   ptx::cluster_sync();
@@ -128,7 +131,7 @@ conv_tc_halo2_kernel(const __grid_constant__ CUtensorMap tm_hi, const __grid_con
   const int num_items = groups * p.n_tiles;
   const int cluster_id = blockIdx.x >> 1;
   const int num_clusters = gridDim.x >> 1;
-  const int nseg = p.h2_nseg;                         // fp32-promotion segments per tile (kH2SegEnd flags of the table)
+  const int nseg = p.h2_nseg;                         // fp32-promotion segments per tile (same rule as seg_end below)
   const int nslots = nseg + (NPLANES == 2 ? 1 : 0);   // accumulation slots (= promotions) per tile
 
   if (warp < kEpiWarp0) {
@@ -162,8 +165,7 @@ conv_tc_halo2_kernel(const __grid_constant__ CUtensorMap tm_hi, const __grid_con
       // ============================== TMA producer: weight halves (both CTAs) ==============================
       if (lane == 0) {
         ptx::prefetch_tensormap(&tm_w);
-        // rows of one (tile, rank) block in the packed weights: 128-byte rows, or 1024-byte rows of the wide map
-        const int wrows = wide_w ? (NPLANES * half_rows) >> 3 : NPLANES * half_rows;
+        const int wrows = NPLANES * half_rows;               // rows of one (tile, rank) block in the packed weights
         int b = 0;
         uint32_t phb = 0;
         for (int item = cluster_id; item < num_items; item += num_clusters) {
@@ -189,8 +191,6 @@ conv_tc_halo2_kernel(const __grid_constant__ CUtensorMap tm_hi, const __grid_con
       // bit b of `phm` = completed uses of buffer b mod 2 (mbarrier phase parity).  Plain increments and selects instead
       // of slot % nbuf keep all of it in uniform registers.
       uint32_t bd = 0, bc = 0, phm = 0;
-      // chunks with the regular one-tap-per-stage layout (all of them unless the packing experiment is on)
-      const int n_reg = p.h2_nreg;
       const int seg_target = 12 * p.seg_chunks;             // promotion period in 16-channel slices (12 = one full (chunk, dx) unit)
 #ifdef DCSCN_H2_DEBUG
       long long w_a = 0, w_b = 0, w_acc = 0;
@@ -203,13 +203,13 @@ conv_tc_halo2_kernel(const __grid_constant__ CUtensorMap tm_hi, const __grid_con
         bool seg_open = true;
         uint32_t tmem_d = 0, tmem_c = 0, acc_d0 = 0;
         bool fresh = true;                                  // the next UMMA slice opens the segment's accumulation slots
-        int st = 0;                                         // stage counter (= index into the table)
+        int st = 0;                                         // weight stage of the item
 
-        // ---- regular part: full 64-channel chunks, one stage per tap, taps in (dx, dy) order, structure known at
-        // compile time (no table reads, dy unrolled): the path almost every UMMA of a layer takes
-        for (int ch = 0; ch < n_reg; ++ch) {
+        // one stage per tap, taps in (dx, dy) order, dy unrolled
+        for (int ch = 0; ch < p.chunks; ++ch) {
           const int kt = min(4, (p.cin_pad - (ch << 6)) >> 4);      // 16-channel slices per tap (3 in a 48-channel tail)
           { H2_T0(); ptx::mbar_wait(&a_full[sa], spa); H2_ACC(w_a); }   // the chunk's halo box serves all nine taps
+          // low descriptor word (start address >> 4 | LBO) of the A slot's hi plane; slots are 1024-byte aligned
           const uint32_t a_desc0 = (((sa_u32 + (uint32_t)sa * (uint32_t)A_SLOT) & 0x3FFFFu) >> 4) | (1u << 16);
           for (int dx = 0; dx < 3; ++dx) {
             if (seg_open) {
@@ -218,11 +218,11 @@ conv_tc_halo2_kernel(const __grid_constant__ CUtensorMap tm_hi, const __grid_con
               tmem_d = tmem_base + bd * (uint32_t)acc_stride;
               tmem_c = tmem_base + bc * (uint32_t)acc_stride;
               fresh = true;
-              acc_d0 = (NPLANES == 2 && s > 0) ? 1u : 0u;
+              acc_d0 = (NPLANES == 2 && s > 0) ? 1u : 0u;     // the dominant slot already holds the previous corrections
               seg_open = false;
             }
             dom += 12;
-            const bool seg_end = (dom >= seg_target) || (st + 3 == nst);   // same rule as build_h2_stages
+            const bool seg_end = (dom >= seg_target) || (st + 3 == nst);   // same rule as h2_segments in engine.cu
 #pragma unroll
             for (int dy = 0; dy < 3; ++dy, ++st) {
               if (!resident || item == cluster_id) { H2_T0(); ptx::mbar_wait(&b_full[sb], spb); H2_ACC(w_b); }   // resident stages landed during the first item
@@ -232,7 +232,7 @@ conv_tc_halo2_kernel(const __grid_constant__ CUtensorMap tm_hi, const __grid_con
               uint32_t ah = a_desc0 + (uint32_t)(dy * kHalo1W + dx) * 8u;
               uint32_t al = ah + (uint32_t)(AH_BYTES >> 4);
               if (ptx::elect_one()) {
-                constexpr uint32_t kDescHiA = (uint32_t)((kHalo1W * 128) >> 4) | (1u << 14) | (2u << 29);
+                constexpr uint32_t kDescHiA = (uint32_t)((kHalo1W * 128) >> 4) | (1u << 14) | (2u << 29);   // SBO 1280, SW128, base offset 0
                 constexpr uint32_t kDescHiB = (uint32_t)(TcSmem<KC>::kSbo >> 4) | (1u << 14) | ((uint32_t)TcSmem<KC>::kLayout << 29);
                 // slice 0 may open the segment's accumulation slots; slices 1.. always accumulate.  Full chunks (kt == 4)
                 // run the remaining slices as straight-line code: the single issuing thread spends ~7 instructions per
@@ -280,7 +280,7 @@ conv_tc_halo2_kernel(const __grid_constant__ CUtensorMap tm_hi, const __grid_con
               fresh = false;
               __syncwarp();
               if (resident) {
-                ++sb;
+                ++sb;                                             // stage st lives in ring slot st; phase 0 stays complete
               } else if (++sb == num_b) {
                 sb = 0;
                 spb ^= 1;
@@ -290,87 +290,11 @@ conv_tc_halo2_kernel(const __grid_constant__ CUtensorMap tm_hi, const __grid_con
               ++s;
               dom = 0;
               seg_open = true;
-              phm ^= 1u << bd;
+              phm ^= 1u << bd;                                // this use of the dominant buffer is complete
               bd = bc;
             }
           }
           if (++sa == num_a) { sa = 0; spa ^= 1; }
-        }
-
-        // ---- tail chunk (cin_pad % 64 channels): table-driven, several taps may share one packed stage
-        for (; st < nst; ++st) {
-          const uint32_t e = s_tab[2 * st];
-          uint32_t rows = s_tab[2 * st + 1];                        // 8 bits per tap: first halo-box row of the tap
-          const int ntaps = (int)((e >> 8) & 15u), kt = (int)((e >> 16) & 15u);
-          if (seg_open) {
-            bc = (bd + 1u == nbuf) ? 0u : bd + 1u;
-            if (NPLANES == 2) ptx::mbar_wait(&acc_empty[bc], ((phm >> bc) & 1u) ^ 1u);
-            tmem_d = tmem_base + bd * (uint32_t)acc_stride;
-            tmem_c = tmem_base + bc * (uint32_t)acc_stride;
-            fresh = true;                                           // corrections open their slot with the first slice
-            acc_d0 = (NPLANES == 2 && s > 0) ? 1u : 0u;             // the dominant slot already holds the previous corrections
-            seg_open = false;
-          }
-          if (e & kH2ChunkFirst) ptx::mbar_wait(&a_full[sa], spa);  // the chunk's halo box serves all its stages
-          if (!resident || item == cluster_id) ptx::mbar_wait(&b_full[sb], spb);
-          ptx::tc_fence_after();
-          // low descriptor word (start address >> 4 | LBO) of the A slot's hi plane; slots are 1024-byte aligned
-          const uint32_t a_desc0 = (((sa_u32 + (uint32_t)sa * (uint32_t)A_SLOT) & 0x3FFFFu) >> 4) | (1u << 16);
-          const uint32_t b_addr = sb_u32 + (uint32_t)sb * (uint32_t)B_STAGE;
-          const uint32_t lb_hi = desc_lo_t<KC>(b_addr), lb_lo = desc_lo_t<KC>(b_addr + BH_BYTES);
-          if (ptx::elect_one()) {
-            // Descriptors are advanced by plain adds on their low words (start address >> 4, 16-byte units): +2 per
-            // 16-channel slice.  The single issuing thread is the scarce resource here - every scalar instruction between
-            // two UMMAs is time the tensor pipe's queue is not being fed (thin layers: 16-32 cycles per UMMA).
-            constexpr uint32_t kDescHiA = (uint32_t)((kHalo1W * 128) >> 4) | (1u << 14) | (2u << 29);          // SBO 1280, SW128
-            constexpr uint32_t kDescHiB = (uint32_t)(TcSmem<KC>::kSbo >> 4) | (1u << 14) | ((uint32_t)TcSmem<KC>::kLayout << 29);
-            uint32_t bh = lb_hi, bl = lb_lo;                        // weight slices walk through the stage's 128-byte rows
-#pragma unroll 1
-            for (int j = 0; j < ntaps; ++j, rows >>= 8) {
-              uint32_t ah = a_desc0 + (rows & 255u) * 8u;           // 128-byte rows = 8 descriptor units each
-              uint32_t al = ah + (uint32_t)(AH_BYTES >> 4);
-#pragma unroll 1
-              for (int ks = 0; ks < kt; ++ks) {
-                const uint64_t da_hi = ((uint64_t)kDescHiA << 32) | ah, db_hi = ((uint64_t)kDescHiB << 32) | bh;
-                if (fresh) {                                        // first slice of a segment: the slots may be opened here
-                  if (NPLANES == 2) {
-                    ptx::mma_f16_ss_2sm(tmem_c, ((uint64_t)kDescHiA << 32) | al, db_hi, idesc, 0);
-                    ptx::mma_f16_ss_2sm_acc(tmem_c, da_hi, ((uint64_t)kDescHiB << 32) | bl, idesc);
-                  }
-                  ptx::mma_f16_ss_2sm(tmem_d, da_hi, db_hi, idesc, acc_d0);
-                  fresh = false;
-                } else {
-                  if (NPLANES == 2) {
-                    ptx::mma_f16_ss_2sm_acc(tmem_c, ((uint64_t)kDescHiA << 32) | al, db_hi, idesc);
-                    ptx::mma_f16_ss_2sm_acc(tmem_c, da_hi, ((uint64_t)kDescHiB << 32) | bl, idesc);
-                  }
-                  ptx::mma_f16_ss_2sm_acc(tmem_d, da_hi, db_hi, idesc);
-                }
-                ah += 2; al += 2; bh += 2; bl += 2;
-              }
-            }
-            if (!resident) ptx::mma_commit_2sm(&b_empty[sb], 3);
-            if (e & kH2ChunkLast) ptx::mma_commit_2sm(&a_empty[sa], 3);
-            if (e & kH2SegEnd) {
-              ptx::mma_commit_2sm(&acc_full[bd], 3);
-              if (NPLANES == 2 && s == nseg - 1) ptx::mma_commit_2sm(&acc_full[bc], 3);
-            }
-          }
-          fresh = false;                                          // (set by the elected lane; every stage has >= 1 slice)
-          __syncwarp();
-          if (resident) {
-            ++sb;                                             // stage st lives in ring slot st; phase 0 stays complete
-          } else if (++sb == num_b) {
-            sb = 0;
-            spb ^= 1;
-          }
-          if ((e & kH2ChunkLast) && ++sa == num_a) { sa = 0; spa ^= 1; }
-          if (e & kH2SegEnd) {
-            ++s;
-            seg_open = true;
-            phm ^= 1u << bd;                                        // this use of the dominant buffer is complete
-            bd = bc;
-          }
         }
         if (NPLANES == 2) {                                         // the corrections-only slot of the last segment
           phm ^= 1u << bd;

@@ -1,7 +1,7 @@
-// CTA-pair variant of the tcgen05 implicit-GEMM convolution (see conv_tc.cuh for the single-CTA description).
+// CTA-pair tcgen05 implicit-GEMM convolution (see conv_tc.cuh for what the tensor-core kernels share).
 //
-// Measured on B200 (profiles/r1a_*): the single-CTA kernel is bound by bytes entering each SM (TMA -> shared memory,
-// ~28 B/clk/SM) - every 128-pixel tile streams the whole layer's weight tiles - not by the tensor pipe (25 % active).
+// Measured on B200 (profiles/r1a_*): a single-CTA form of this kernel was bound by bytes entering each SM (TMA -> shared
+// memory, ~28 B/clk/SM) - every 128-pixel tile streams the whole layer's weight tiles - not by the tensor pipe (25 % active).
 // Here two CTAs of one TPC form a cluster and issue `tcgen05.mma.cta_group::2` with M = 256 (two 128-pixel tiles):
 // each CTA stages only HALF of every weight tile (N/2 rows) and the tensor core reads the other half from the
 // peer's shared memory, so weight bytes per SM (and weight shared-memory reads) are halved.

@@ -21,8 +21,6 @@
 #include "conv_aux.cuh"
 #include "conv_tc.cuh"
 #include "conv_tc_pair.cuh"
-#include "conv_tc_halo.cuh"
-#include "conv_tc_halo1.cuh"
 #include "conv_tc_halo2.cuh"
 #include "conv_ds.cuh"
 #include "conv_ds_tile.cuh"
@@ -86,23 +84,15 @@ struct TcLayer {
   std::vector<float> bias_host, alpha_host;  // [n_tiles*n_pad]
   int cin = 0, cout = 0;
   float wscale = 1.f;
-  __half* d_wpack = nullptr;
   float* d_bias = nullptr;
   float* d_alpha = nullptr;
   float* d_wref = nullptr;      // fp32 HWIO for the validation kernel
   int* d_in_map = nullptr;
-  int packed_kc = 0, packed_planes = 0;
-  __half* d_wpair = nullptr;    // CTA-pair layout [n_tile][tap][chunk][rank][plane][n_pad/2 x 64]
+  __half* d_wpair = nullptr;    // CTA-pair layout [n_tile][block][rank][plane][n_pad/2 x 64], blocks as in pair_image
   CUtensorMap tm_w;             // 2-D map over d_wpair (rows of 128 bytes)
-  CUtensorMap tm_w_wide;        // the same bytes as rows of 1024 bytes (fp32 elements, no swizzle): fewer, longer TMA rows
-  bool has_wide = false;
-  bool has_pair = false;
-  // streaming 3x3 kernel: weight-stage table of one item (conv_tc_halo2.cuh); non-empty = d_wpair is in stage order
-  std::vector<uint32_t> h2_stages;
-  int h2_nseg = 0;
-  int h2_nreg = 0;                  // leading chunks with one tap per stage
-  int h2_seg_units = 1;             // promotion period of the regular (full-chunk) part, in (chunk, dx) units
-  uint32_t* d_h2_stages = nullptr;
+  bool h2 = false;              // streaming 3x3 kernel (conv_tc_halo2.cuh): d_wpair is in its [chunk][dx][dy] stage order
+  int h2_nseg = 0;              // its fp32-promotion segments per item
+  int h2_seg_units = 1;         // its promotion period, in (chunk, dx) units
   int* d_pair_src = nullptr;    // training: flat parameter index behind every hi-plane element of d_wpair (-1 = zero)
   size_t pair_src_n = 0;
 };
@@ -117,29 +107,17 @@ struct TcLaunch {
   int layer_index = -1;          // index into dcscn_handle::tcl (forward) or ::bwd (dgrad twins): the layer whose CURRENT
   bool layer_bwd = false;        // power-of-two weight scale the epilogue has to undo (it changes when a layer is re-packed)
   CUtensorMap tm_hi, tm_lo, tm_w;
-  bool pair = false;
   int pair_grid = 0, pair_stages = 0, pair_seg = 1;
   bool pair_stream = false;
-  bool halo = false;             // 3x3 layers: halo-reuse CTA-pair kernel
-  CUtensorMap th_hi, th_lo;      // A maps with box {64, 8, 18, 1}
+  size_t pair_smem = 0;
+  bool halo2 = false;            // 3x3 layers: streaming halo kernel on 16 x 8 pixel patches
   ConvGeom hg;
-  int halo_grid = 0, halo_na = 0, halo_nb = 0, halo_seg = 1;
-  size_t halo_smem = 0;
-  bool halo1 = false;            // single 10 x 18 halo box per chunk serves all nine taps (default for 3x3 layers)
-  CUtensorMap t1_hi, t1_lo;
-  int halo1_na = 0, halo1_nb = 0, halo1_seg = 1;
-  size_t halo1_smem = 0;
-  CUtensorMap tm_w_wide;
-  bool has_wide = false;
-  bool halo2 = false;            // streaming halo kernel (split correction / dominant accumulators), default
+  int halo_grid = 0;
+  CUtensorMap t1_hi, t1_lo;      // A maps with box {64, 10, 18, 1}
   int halo2_na = 0, halo2_nb = 0, halo2_seg = 1;
   size_t halo2_smem = 0;
-  size_t pair_smem = 0;
   ConvTCParams p;
   ConvRefParams ref;
-  int grid = 0;
-  int stages = 0;
-  size_t smem = 0;
 };
 
 struct Plan {
@@ -192,7 +170,6 @@ struct dcscn_handle {
   double* ensio_y = nullptr;
   size_t ensio_cap = 0;
   int l1_loss = 0;                   // --use_l1_loss: image_loss = mean |y_ - y| (DCSCN.py:342-344)
-  int wgrad_halo = 1;                // the three dx taps of a filter row share one 18-pixel-wide A box
   int wgrad_taps = 0;                // 0 = automatic (up to 3 filter taps per wgrad CTA), else the cap
   int wgrad_impl = 0;                // 0 = tcgen05 (wgrad_tc.cuh), 1 = CUDA cores (validation)
   int host_repack = 0;               // option: always re-pack on the host after an update (validation of the device path)
@@ -253,15 +230,8 @@ struct dcscn_handle {
   int64_t graph_replays = 0;
 
   int conv_impl = 0;
-  int kc = 64;
   int seg_chunks = 0;                // pipeline stages per fp32-promotion segment; 0 = automatic
   int act_grad_impl = 0;             // 0: 16-byte activation-gradient kernel, 1: channel-pair kernel (cross-check)
-  int cluster = 1;                   // CTAs per cluster multicasting the weight tiles (single-CTA kernel)
-  int pair = 1;                      // use the CTA-pair (tcgen05 cta_group::2) kernel when KC == 64
-  int halo = 3;                      // 3x3 layers: halo-reuse CTA-pair kernel, 1 = three 18x8 boxes, 2 = one 18x10 box per chunk
-                                     // (two-pass segments), 3 = the same box with streaming stages (conv_tc_halo2.cuh)
-  int halo_base = 0;                 // single-box variant: set the descriptor base-offset field
-  int wmap_wide = 0;                 // streaming kernel: fetch weight stages as rows of 1024 bytes instead of 128
   int timing = 0;
   int fuse_last = 1;                 // fold the per-pixel half of R-CNN1 into the last Up-PS epilogue
   std::vector<cudaEvent_t> ev;       // timing events (launch boundaries of the last forward)
@@ -424,14 +394,12 @@ static void choose_tiling(int n_total_pad16, int* n_tiles, int* n_pad, int cap =
   *n_pad = np;
 }
 
-// Values (unscaled fp32) of the CTA-pair operand image of a layer, one per hi-plane element, in image order:
-// [n_tile][tap][chunk][rank][n_pad/2 rows x 64 halves], each row 128-byte swizzled (16-byte chunk j of row r at j ^ (r & 7)).
-static int tile_cap(const dcscn_handle* h, int ksz);
-static bool streaming3x3(const dcscn_handle* h);
+// Column-tile cap of a layer.  The streaming 3x3 kernel rotates TMEM buffers of n_pad columns: 160 keeps three of them
+// (3 * n_pad <= 512).  Option "wide_tiles" lifts it to 256: layers wider than 160 columns then run with TWO buffers (the
+// issuer waits for a drain at every segment end) but read every A box once per pixel tile instead of once per column
+// tile - CNN2 is one tile of 176 columns instead of 2 x 96, Up-PS 2 x 192 instead of 4 x 96.
+static int tile_cap(const dcscn_handle* h, int ksz) { return ksz == 3 ? (h->wide_tiles ? 256 : 160) : 256; }
 
-// Weight-stage table of the streaming 3x3 kernel (see conv_tc_halo2.cuh): full 64-channel chunks take one stage per tap,
-// a last chunk with 16 / 32 valid channels packs 4 / 2 taps per stage.  `seg_units` = promotion period in units of 12
-// dominant UMMAs (3 taps x 4 slices), like the (chunk, dx) units of the two-pass kernels.
 // Experiments: DCSCN_SEG="CNN2=1,A1=6" overrides the fp32-promotion period of single layers.
 static int seg_override(const std::string& name, int seg) {
   if (const char* ov = getenv("DCSCN_SEG")) {
@@ -442,90 +410,18 @@ static int seg_override(const std::string& name, int seg) {
   return std::max(1, seg);
 }
 
-static void build_h2_stages(int cin_pad, int seg_units, std::vector<uint32_t>& tab, int* nseg, int* nreg) {
-  tab.clear();
-  // Packing several taps of a 16/32-channel tail chunk into one 64-half stage saves weight stages but sends those stages
-  // through the table-driven issue loop; measured on B200 it loses (B2 0.122 -> 0.151 ms, CNN9 0.248 -> 0.306 ms), so it
-  // is an experiment switch only.
-  static const bool pack_tails = getenv("DCSCN_H2_PACK") && atoi(getenv("DCSCN_H2_PACK")) == 1;
-  *nreg = 0;
-  const int chunks = (cin_pad + 63) / 64, target = 12 * std::max(1, seg_units);
-  int dom = 0, segs = 0;
-  for (int ch = 0; ch < chunks; ++ch) {
-    const int kt = std::min(64, cin_pad - ch * 64) / 16;            // 16-channel slices per tap in this chunk (1..4)
-    const int per = (kt >= 3 || !pack_tails) ? 1 : 4 / kt;          // taps per stage
-    if (per == 1 && *nreg == ch) *nreg = ch + 1;
-    for (int t0 = 0; t0 < 9; t0 += per) {
-      const int nt = std::min(per, 9 - t0);
-      uint32_t e = (uint32_t)ch | ((uint32_t)nt << 8) | ((uint32_t)t0 << 12) | ((uint32_t)kt << 16);
-      uint32_t rows = 0;                                           // first halo-box row (dy * 10 + dx) of each tap, 8 bits each
-      for (int j = 0; j < nt; ++j) {
-        const int tap = t0 + j, dx = tap / 3, dy = tap % 3;
-        rows |= (uint32_t)(dy * kHalo1W + dx) << (8 * j);
-      }
-      if (t0 == 0) e |= kH2ChunkFirst;
-      if (t0 + nt >= 9) e |= kH2ChunkLast;
-      dom += (per == 1) ? 4 : nt * kt;                            // a one-tap stage counts as a full one whatever its kt
-      const bool last = (ch == chunks - 1) && (t0 + nt >= 9);
-      // one-tap stages end a segment only after a whole (chunk, dx) unit: the kernel's regular path issues those three
-      // stages as one block
-      const bool boundary = (per > 1) || (t0 % 3 == 2);
-      if ((dom >= target && boundary) || last) {
-        e |= kH2SegEnd;
-        dom = 0;
-        ++segs;
-      }
-      tab.push_back(e);
-      tab.push_back(rows);
-    }
-  }
-  *nseg = segs;
+// fp32-promotion segments of one item of the streaming 3x3 kernel: a segment ends after `seg_units` (chunk, dx) units of
+// 12 dominant UMMAs (3 taps x 4 slices), or with the last unit - the rule of the kernel's seg_end.
+static int h2_segments(int cin_pad, int seg_units) {
+  const int units = 3 * ((cin_pad + 63) / 64);
+  return (units + seg_units - 1) / seg_units;
 }
 
-// Stage-ordered operand image of the streaming kernel: [n_tile][stage][rank][n_pad/2 rows x 64 halves]; the four
-// 16-channel slices of a row belong to (tap0 + q / kt, slice q % kt) of the stage's chunk.
-static void pair_image_h2(const TcLayer& t, std::vector<float>& img) {
-  const int n_total = t.n_tiles * t.n_pad, nst = (int)t.h2_stages.size() / 2;
-  std::vector<float> wq((size_t)9 * t.cin_pad * n_total, 0.f);     // dense, channel-position-indexed  Wq[tap][q][n]
-  for (int tp = 0; tp < 9; ++tp)
-    for (int ci = 0; ci < t.cin; ++ci) {
-      const int q = t.in_map[ci];
-      for (int co = 0; co < t.cout; ++co)
-        wq[((size_t)tp * t.cin_pad + q) * n_total + co] = t.w_host[((size_t)tp * t.cin + ci) * t.cout + co];
-    }
-  const int half_rows = t.n_pad / 2;
-  const size_t half_elems = (size_t)half_rows * 64;
-  img.assign((size_t)t.n_tiles * nst * 2 * half_elems, 0.f);
-  for (int nt = 0; nt < t.n_tiles; ++nt)
-    for (int st = 0; st < nst; ++st) {
-      const uint32_t e = t.h2_stages[2 * st];
-      const int ch = (int)(e & 255u), ntaps = (int)((e >> 8) & 15u), tap0 = (int)((e >> 12) & 15u), kt = (int)((e >> 16) & 15u);
-      for (int rk = 0; rk < 2; ++rk) {
-        float* base = img.data() + (((size_t)nt * nst + st) * 2 + rk) * half_elems;
-        for (int r = 0; r < half_rows; ++r) {
-          const int n = nt * t.n_pad + rk * half_rows + r;
-          const int sw = r & 7;
-          for (int col = 0; col < ntaps * kt; ++col) {
-            const int tap = tap0 + col / kt, ks = col % kt;
-            const int dx = tap / 3, dy = tap % 3;                   // table order is dx-major; HWIO taps are ky * 3 + kx
-            const int hwio_tap = dy * 3 + dx;
-            for (int e16 = 0; e16 < 16; ++e16) {
-              const int q = ch * 64 + ks * 16 + e16;
-              if (q >= t.cin_pad) continue;
-              const int kk = col * 16 + e16;
-              base[(size_t)r * 64 + (size_t)((kk / 8) ^ sw) * 8 + (kk % 8)] = wq[((size_t)hwio_tap * t.cin_pad + q) * n_total + n];
-            }
-          }
-        }
-      }
-    }
-}
-
+// Values (unscaled fp32) of the CTA-pair operand image of a layer, one per hi-plane element, in image order:
+// [n_tile][block][rank][n_pad/2 rows x 64 halves], each row 128-byte swizzled (16-byte chunk j of row r at j ^ (r & 7)).
+// A block holds one filter tap of one 64-channel chunk.  Blocks are in [tap][chunk] order for conv_tc_pair_kernel, and in
+// the streaming kernel's stage order [chunk][dx][dy] when t.h2 is set.
 static void pair_image(const TcLayer& t, std::vector<float>& img) {
-  if (!t.h2_stages.empty()) {
-    pair_image_h2(t, img);
-    return;
-  }
   const int taps = t.ksz * t.ksz, chunks = (t.cin_pad + 63) / 64, n_total = t.n_tiles * t.n_pad;
   std::vector<float> wq((size_t)taps * t.cin_pad * n_total, 0.f);   // dense, channel-position-indexed  Wq[tap][q][n]
   for (int tp = 0; tp < taps; ++tp)
@@ -539,9 +435,11 @@ static void pair_image(const TcLayer& t, std::vector<float>& img) {
   img.assign((size_t)t.n_tiles * taps * chunks * 2 * half_elems, 0.f);
   for (int nt = 0; nt < t.n_tiles; ++nt)
     for (int tp = 0; tp < taps; ++tp)
-      for (int ch = 0; ch < chunks; ++ch)
+      for (int ch = 0; ch < chunks; ++ch) {
+        // HWIO tap tp = dy * 3 + dx is stage dx * 3 + dy of its chunk in the streaming order
+        const int blk = t.h2 ? ch * 9 + (tp % 3) * 3 + tp / 3 : tp * chunks + ch;
         for (int rk = 0; rk < 2; ++rk) {
-          float* base = img.data() + ((((size_t)nt * taps + tp) * chunks + ch) * 2 + rk) * half_elems;
+          float* base = img.data() + (((size_t)nt * taps * chunks + blk) * 2 + rk) * half_elems;
           for (int r = 0; r < half_rows; ++r) {
             const int n = nt * t.n_pad + rk * half_rows + r;
             const int sw = r & 7;
@@ -551,60 +449,20 @@ static void pair_image(const TcLayer& t, std::vector<float>& img) {
             }
           }
         }
+      }
 }
 
 static int pack_tc_layer(dcscn_handle* h, TcLayer& t) {
-  const int KC = h->kc;
   const int NPL = planes(h);
-  const int taps = t.ksz * t.ksz;
-  const int chunks = (t.cin_pad + KC - 1) / KC;
-  const int n_total = t.n_tiles * t.n_pad;
 
   float maxw = 0.f;
   for (float v : t.w_host) maxw = std::max(maxw, std::fabs(v));
   t.wscale = 1.f;
   if (maxw > 0.f) t.wscale = std::ldexp(1.0f, (int)std::floor(std::log2(16384.0 / (double)maxw)));
 
-  const int row_chunks = KC / 8;
-  const size_t tile_elems = (size_t)t.n_pad * KC;
-  const bool need_pair = (KC == 64) && h->pair && (h->sm_count % 2 == 0);
-  const bool need_single = !need_pair;   // the single-CTA kernel only runs when the CTA-pair kernels cannot
-  // dense, channel-position-indexed weights  Wq[tap][q][n]
-  std::vector<float> wq(need_single ? (size_t)taps * t.cin_pad * n_total : 0, 0.f);
-  for (int tp = 0; need_single && tp < taps; ++tp)
-    for (int ci = 0; ci < t.cin; ++ci) {
-      const int q = t.in_map[ci];
-      for (int co = 0; co < t.cout; ++co)
-        wq[((size_t)tp * t.cin_pad + q) * n_total + co] = t.w_host[((size_t)tp * t.cin + ci) * t.cout + co] * t.wscale;
-    }
-
-  // tiles in the shared-memory image of a K-major swizzled UMMA operand: row = output channel, KC halves per row,
-  // 16-byte chunk j of row r lands at chunk j ^ f(r)  (SW128: f = r & 7, SW64: f = (r >> 1) & 3)
-  std::vector<__half> pack(need_single ? (size_t)t.n_tiles * taps * chunks * NPL * tile_elems : 0);
-  for (int nt = 0; need_single && nt < t.n_tiles; ++nt)
-    for (int tp = 0; tp < taps; ++tp)
-      for (int ch = 0; ch < chunks; ++ch) {
-        __half* base = pack.data() + (((size_t)nt * taps + tp) * chunks + ch) * NPL * tile_elems;
-        for (int r = 0; r < t.n_pad; ++r) {
-          const int n = nt * t.n_pad + r;
-          const int sw = (KC == 64) ? (r & 7) : ((r >> 1) & 3);
-          for (int kk = 0; kk < KC; ++kk) {
-            const int q = ch * KC + kk;
-            float v = (q < t.cin_pad) ? wq[((size_t)tp * t.cin_pad + q) * n_total + n] : 0.f;
-            __half hi = __float2half_rn(v);
-            __half lo = __float2half_rn(v - __half2float(hi));
-            const int j = kk / 8, e = kk % 8;
-            const size_t pos = (size_t)r * KC + (size_t)((j ^ sw) % row_chunks) * 8 + e;
-            base[pos] = hi;
-            if (NPL == 2) base[tile_elems + pos] = lo;
-          }
-        }
-      }
-  if (upload(&t.d_wpack, pack, h)) return 1;
-  t.has_pair = false;
-  t.h2_stages.clear();
+  t.h2 = t.ksz == 3 && (h->wide_tiles ? 2 : 3) * t.n_pad <= 512;   // streaming kernel: stage-ordered image
   t.h2_nseg = 0;
-  if (need_pair && t.ksz == 3 && streaming3x3(h) && (h->wide_tiles ? 2 : 3) * t.n_pad <= 512) {   // streaming kernel: stage-ordered image
+  if (t.h2) {
     // Promotion period in (chunk, dx) units of K = 192.  Measured (gpurun_out/seg15.log): with three TMEM buffers
     // (n_pad >= 144) a period of 1 leaves the epilogue one segment (~1.5 us) to drain a slot and the issuer stalls -
     // CNN3 0.85 -> 0.63 ms, CNN4 0.74 -> 0.52 ms at 4; the noise-tile error is flat in this range (1.2-1.35e-3).
@@ -612,63 +470,35 @@ static int pack_tc_layer(dcscn_handle* h, TcLayer& t) {
     // pays twice there: CNN2 as one 176-column tile 0.93 -> 0.88 ms at 4 units, noise-tile error unchanged (1.27 -> 1.28e-3).
     const int seg = seg_override(t.name, h->seg_chunks > 0 ? h->seg_chunks : (t.n_pad >= 144 ? 4 : 3));
     t.h2_seg_units = seg;
-    build_h2_stages(t.cin_pad, seg, t.h2_stages, &t.h2_nseg, &t.h2_nreg);
-    if ((int)t.h2_stages.size() / 2 > kH2MaxTable) return fail("layer %s: %zu weight stages exceed the kernel's table", t.name.c_str(), t.h2_stages.size());
-    if (upload(&t.d_h2_stages, t.h2_stages, h)) return 1;
+    t.h2_nseg = h2_segments(t.cin_pad, seg);
   }
-  if (need_pair) {
-    const int half_rows = t.n_pad / 2;
-    const size_t half_elems = (size_t)half_rows * 64;
-    std::vector<float> img;
-    pair_image(t, img);
-    std::vector<__half> pp(img.size() * NPL);
-    for (size_t i = 0; i < img.size(); ++i) {
-      const size_t blk = i / half_elems, pos = i - blk * half_elems;
-      const float v = img[i] * t.wscale;
-      const __half hi = __float2half_rn(v);
-      pp[blk * NPL * half_elems + pos] = hi;
-      if (NPL == 2) pp[blk * NPL * half_elems + half_elems + pos] = __float2half_rn(v - __half2float(hi));
-    }
-    if (upload(&t.d_wpair, pp, h)) return 1;
-    const size_t total_rows = pp.size() / 64;
-    cuuint64_t dims[2] = {64, (cuuint64_t)total_rows};
-    cuuint64_t strides[1] = {128};
-    cuuint32_t box[2] = {64, (cuuint32_t)(NPL * half_rows)};
-    cuuint32_t estr[2] = {1, 1};
-    CUresult r = h->encode(&t.tm_w, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, (void*)t.d_wpair, dims, strides, box, estr,
-                           CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                           CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) return fail("cuTensorMapEncodeTiled (weights, layer %s) failed: %d", t.name.c_str(), (int)r);
-    t.has_pair = true;
-    t.has_wide = false;
-    const size_t stage_bytes = (size_t)NPL * half_rows * 128;
-    if (stage_bytes % 1024 == 0 && stage_bytes / 1024 <= 256) {
-      cuuint64_t wdims[2] = {256, (cuuint64_t)(pp.size() * 2 / 1024)};
-      cuuint64_t wstrides[1] = {1024};
-      cuuint32_t wbox[2] = {256, (cuuint32_t)(stage_bytes / 1024)};
-      r = h->encode(&t.tm_w_wide, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, (void*)t.d_wpair, wdims, wstrides, wbox, estr,
-                    CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                    CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-      t.has_wide = (r == CUDA_SUCCESS);
-    }
+  const int half_rows = t.n_pad / 2;
+  const size_t half_elems = (size_t)half_rows * 64;
+  std::vector<float> img;
+  pair_image(t, img);
+  std::vector<__half> pp(img.size() * NPL);
+  for (size_t i = 0; i < img.size(); ++i) {
+    const size_t blk = i / half_elems, pos = i - blk * half_elems;
+    const float v = img[i] * t.wscale;
+    const __half hi = __float2half_rn(v);
+    pp[blk * NPL * half_elems + pos] = hi;
+    if (NPL == 2) pp[blk * NPL * half_elems + half_elems + pos] = __float2half_rn(v - __half2float(hi));
   }
+  if (upload(&t.d_wpair, pp, h)) return 1;
+  const size_t total_rows = pp.size() / 64;
+  cuuint64_t dims[2] = {64, (cuuint64_t)total_rows};
+  cuuint64_t strides[1] = {128};
+  cuuint32_t box[2] = {64, (cuuint32_t)(NPL * half_rows)};
+  cuuint32_t estr[2] = {1, 1};
+  CUresult r = h->encode(&t.tm_w, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, (void*)t.d_wpair, dims, strides, box, estr,
+                         CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+                         CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  if (r != CUDA_SUCCESS) return fail("cuTensorMapEncodeTiled (weights, layer %s) failed: %d", t.name.c_str(), (int)r);
   if (upload(&t.d_bias, t.bias_host, h)) return 1;
   if (upload(&t.d_alpha, t.alpha_host, h)) return 1;
   if (upload(&t.d_wref, t.w_host, h)) return 1;
   if (upload(&t.d_in_map, t.in_map, h)) return 1;
-  t.packed_kc = KC;
-  t.packed_planes = NPL;
   return 0;
-}
-
-// Column-tile cap of a layer: the streaming 3x3 kernel rotates three TMEM buffers of n_pad columns (3 * n_pad <= 512).
-static bool streaming3x3(const dcscn_handle* h) { return h->halo == 3 && h->pair && h->kc == 64 && h->sm_count % 2 == 0; }
-// Column-tile cap of the streaming 3x3 kernel: 160 keeps three TMEM buffers (3 * n_pad <= 512).  Option "wide_tiles" lifts
-// it to 256: layers wider than 160 columns then run with TWO buffers (the issuer waits for a drain at every segment end)
-// but read every A box once per pixel tile instead of once per column tile - CNN2 is one tile of 176 columns instead of
-// 2 x 96, Up-PS 2 x 192 instead of 4 x 96.
-static int tile_cap(const dcscn_handle* h, int ksz) {
-  return (ksz == 3 && streaming3x3(h)) ? (h->wide_tiles ? 256 : 160) : 256;
 }
 
 static TcLayer make_tc(const dcscn_handle* h, const std::string& name, int ksz, int cin, int cout_cols, int cin_pad,
@@ -681,7 +511,7 @@ static TcLayer make_tc(const dcscn_handle* h, const std::string& name, int ksz, 
   t.cout = cout_cols;
   t.cin_pad = cin_pad;
   choose_tiling(pad16(cout_cols), &t.n_tiles, &t.n_pad, cap);
-  if (tile_unit > 0 && cap < 256 && ksz == 3 && streaming3x3(h) && t.n_tiles > 1 && tile_unit % 16 == 0 && tile_unit <= cap && cout_cols % tile_unit == 0) {
+  if (tile_unit > 0 && cap < 256 && ksz == 3 && t.n_tiles > 1 && tile_unit % 16 == 0 && tile_unit <= cap && cout_cols % tile_unit == 0) {
     t.n_pad = tile_unit;               // pixel-shuffler layers: one column tile per sub-pixel (fused R-CNN1 epilogue)
     t.n_tiles = cout_cols / tile_unit;
   }
@@ -693,24 +523,21 @@ static TcLayer make_tc(const dcscn_handle* h, const std::string& name, int ksz, 
 }
 
 static void free_tc(TcLayer& t) {
-  dev_free(t.d_wpack);
   dev_free(t.d_wpair);
   dev_free(t.d_bias);
   dev_free(t.d_alpha);
   dev_free(t.d_wref);
   dev_free(t.d_in_map);
   dev_free(t.d_pair_src);
-  dev_free(t.d_h2_stages);
-  t.d_h2_stages = nullptr;
   t.d_pair_src = nullptr;
-  t.d_wpack = t.d_wpair = nullptr;
+  t.d_wpair = nullptr;
   t.d_bias = t.d_alpha = t.d_wref = nullptr;
   t.d_in_map = nullptr;
 }
 
 static void adopt_tc(TcLayer& t, const TcLayer& old) {  // keep the device allocations of the previous packing
-  t.d_wpack = old.d_wpack; t.d_wpair = old.d_wpair; t.d_bias = old.d_bias; t.d_alpha = old.d_alpha;
-  t.d_wref = old.d_wref; t.d_in_map = old.d_in_map; t.d_pair_src = old.d_pair_src; t.d_h2_stages = old.d_h2_stages;
+  t.d_wpair = old.d_wpair; t.d_bias = old.d_bias; t.d_alpha = old.d_alpha;
+  t.d_wref = old.d_wref; t.d_in_map = old.d_in_map; t.d_pair_src = old.d_pair_src;
 }
 
 // (Re)builds every device-side weight image from the host fp32 parameters.
@@ -965,15 +792,13 @@ static void choose_patch(int H, int W, int* TH, int* TW) {
 }
 
 static int encode_map(dcscn_handle* h, CUtensorMap* tm, const __half* base, int cin_pad, int pitch, int n, int H,
-                      int W, int TH, int TW, int kc_override = 0) {
-  const int KC = kc_override ? kc_override : h->kc;
+                      int W, int TH, int TW) {
   cuuint64_t dims[4] = {(cuuint64_t)cin_pad, (cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)n};
   cuuint64_t strides[3] = {(cuuint64_t)pitch * 2, (cuuint64_t)W * pitch * 2, (cuuint64_t)H * W * pitch * 2};
-  cuuint32_t box[4] = {(cuuint32_t)KC, (cuuint32_t)TW, (cuuint32_t)TH, 1};
+  cuuint32_t box[4] = {64, (cuuint32_t)TW, (cuuint32_t)TH, 1};
   cuuint32_t estr[4] = {1, 1, 1, 1};
   CUresult r = h->encode(tm, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 4, (void*)base, dims, strides, box, estr,
-                         CU_TENSOR_MAP_INTERLEAVE_NONE,
-                         KC == 64 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_64B,
+                         CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
                          CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   if (r != CUDA_SUCCESS)
     return fail("cuTensorMapEncodeTiled failed (%d) cin_pad=%d pitch=%d n=%d H=%d W=%d box=%dx%d", (int)r, cin_pad,
@@ -997,14 +822,10 @@ static int add_tc_launch(dcscn_handle* h, Plan* pl, const TcLayer& t, const __ha
   L.p.g = g;
   L.p.ksz = t.ksz;
   L.p.cin_pad = t.cin_pad;
-  L.p.chunks = (t.cin_pad + h->kc - 1) / h->kc;
+  L.p.chunks = (t.cin_pad + 63) / 64;
   L.p.n_tiles = t.n_tiles;
   L.p.n_pad = t.n_pad;
-  L.p.seg_chunks = h->seg_chunks;  // finalised per kernel variant below (needs the stage count)
-  int cs = h->cluster;
-  while (cs > 1 && (t.n_pad % cs != 0 || h->sm_count % cs != 0)) cs >>= 1;
-  L.p.cluster_size = cs;
-  L.p.wpack = t.d_wpack;
+  L.p.seg_chunks = h->seg_chunks;  // finalised per kernel at launch
   L.p.epi = epi;
   L.p.epi.bias = t.d_bias;
   L.p.epi.alpha = t.d_alpha;
@@ -1019,119 +840,39 @@ static int add_tc_launch(dcscn_handle* h, Plan* pl, const TcLayer& t, const __ha
   L.p.epi.n_valid = t.n_valid;
   L.p.epi.drop_ntotal = pad16(t.cout);   // keep-mask index stride = slot width, whatever the column tiling
 
-  const size_t stage = tc_stage_bytes(h->kc, planes(h), t.n_pad);
+  // CTA-pair launch shape
   const size_t budget = 227 * 1024 - 2048 - kRdotSmemBytes;
-  int stages = (int)std::min<size_t>(kMaxStages, budget / stage);
-  if (stages < 2) return fail("layer %s: pipeline stage of %zu bytes does not fit twice in shared memory", t.name.c_str(), stage);
-  L.stages = stages;
+  const long long tiles = (long long)n * g.tiles_x * g.tiles_y;
+  L.tm_w = t.tm_w;
+  const size_t pstage = tc_pair_stage_bytes(planes(h), t.n_pad);
+  L.pair_stages = (int)std::min<size_t>(kMaxStages, budget / pstage);
+  if (L.pair_stages < 2) return fail("layer %s: pipeline stage of %zu bytes does not fit twice in shared memory", t.name.c_str(), pstage);
+  L.pair_smem = L.pair_stages * pstage + 1024 + kPairBarBytes + kRdotSmemBytes;
+  const long long pitems = ((tiles + 1) / 2) * t.n_tiles;
+  L.pair_grid = (int)std::min<long long>(pitems, h->sm_count / 2) * 2;
   {
     int seg = h->seg_chunks > 0 ? h->seg_chunks : (t.n_pad >= 112 ? 2 : 3);
-    L.p.seg_chunks = std::max(1, std::min(seg, stages - 1));   // a segment's stages stay resident until its 2nd pass
+    L.pair_seg = std::max(1, std::min(seg, L.pair_stages - 1));   // a segment's stages stay resident until its 2nd pass
   }
-  L.smem = stages * stage + 1024 + 256 + kRdotSmemBytes;
-  const long long tiles = (long long)n * g.tiles_x * g.tiles_y;
-  const long long items = ((tiles + cs - 1) / cs) * t.n_tiles;    // cluster iterations
-  L.grid = (int)std::min<long long>(items, h->sm_count / cs) * cs;
+  // 1x1 layers stream (split accumulators over four TMEM buffers): nothing is held, the promotion period is free
+  L.pair_stream = t.ksz == 1 && planes(h) == 2 && t.n_pad <= kPairStreamStride;
+  if (L.pair_stream) L.pair_seg = seg_override(t.name, h->seg_chunks > 0 ? h->seg_chunks : 4);
 
-  // CTA-pair launch shape
-  L.pair = t.has_pair && (h->sm_count % 2 == 0);
-  if (L.pair) {
-    L.tm_w = t.tm_w;
-    L.tm_w_wide = t.tm_w_wide;
-    L.has_wide = t.has_wide;
-    const size_t pstage = tc_pair_stage_bytes(planes(h), t.n_pad);
-    L.pair_stages = (int)std::min<size_t>(kMaxStages, budget / pstage);
-    L.pair_smem = L.pair_stages * pstage + 1024 + kPairBarBytes + kRdotSmemBytes;
-    const long long pitems = ((tiles + 1) / 2) * t.n_tiles;
-    L.pair_grid = (int)std::min<long long>(pitems, h->sm_count / 2) * 2;
-    if (L.pair_stages < 2) L.pair = false;
-    int seg = h->seg_chunks > 0 ? h->seg_chunks : (t.n_pad >= 112 ? 2 : 3);
-    L.pair_seg = std::max(1, std::min(seg, L.pair_stages - 1));
-    // 1x1 layers stream (split accumulators over four TMEM buffers): nothing is held, the promotion period is free
-    static const bool allow_stream = !(getenv("DCSCN_PAIR_STREAM") && atoi(getenv("DCSCN_PAIR_STREAM")) == 0);   // A/B switch
-    L.pair_stream = allow_stream && t.ksz == 1 && planes(h) == 2 && t.n_pad <= kPairStreamStride;
-    if (L.pair_stream) L.pair_seg = seg_override(t.name, h->seg_chunks > 0 ? h->seg_chunks : 4);
-  }
-
-  // halo-reuse launch shapes (3x3 layers, CTA pair, KC = 64): 16 x 8 pixel patches
-  const bool pair3x3 = L.pair && t.ksz == 3;
-  L.halo = pair3x3;
-  if (pair3x3) {
+  // streaming halo kernel (3x3 layers, 16 x 8 pixel patches): every ring slot is prefetch depth; two, three (n_pad > 128)
+  // or four TMEM accumulation buffers
+  if (t.h2) {
     ConvGeom hg{n, H, W, (W + kHaloTW - 1) / kHaloTW, (H + kHaloTH - 1) / kHaloTH, kHaloTW, kHaloTH};
     L.hg = hg;
     const long long htiles = (long long)n * hg.tiles_x * hg.tiles_y;
     const long long hitems = ((htiles + 1) / 2) * t.n_tiles;
     L.halo_grid = (int)std::min<long long>(hitems, h->sm_count / 2) * 2;
-  }
-  if (L.halo && h->halo == 1) {   // three 18 x 8 boxes per chunk (superseded; kept selectable for A/B runs)
-    if (encode_map(h, &L.th_hi, src_hi, t.cin_pad, src_pitch, n, H, W, kHaloTH + 2, kHaloTW, 64)) return 1;
-    if (planes(h) == 2) {
-      if (encode_map(h, &L.th_lo, src_lo, t.cin_pad, src_pitch, n, H, W, kHaloTH + 2, kHaloTW, 64)) return 1;
-    } else {
-      L.th_lo = L.th_hi;
-    }
-    const size_t a_slot = tc_halo_a_slot_bytes(planes(h)), b_stage = tc_halo_b_stage_bytes(planes(h), t.n_pad);
-    int seg = h->seg_chunks > 0 ? h->seg_chunks : (t.n_pad >= 112 ? 1 : 2);
-    for (;; --seg) {
-      const int na = seg + 2;
-      const long long left = (long long)budget - (long long)na * (long long)a_slot;
-      const int nb = left > 0 ? (int)std::min<long long>(kMaxStages, left / (long long)b_stage) : 0;
-      if (nb >= 3 * seg + 1 && na <= kMaxStages) {
-        L.halo_seg = seg;
-        L.halo_na = na;
-        L.halo_nb = nb;
-        break;
-      }
-      if (seg == 1) {
-        L.halo = false;
-        break;
-      }
-    }
-    if (L.halo) L.halo_smem = L.halo_na * a_slot + L.halo_nb * b_stage + 1024 + 512 + kRdotSmemBytes;
-  } else {
-    L.halo = false;
-  }
-
-  L.halo1 = false;
-  if (pair3x3) {
-    const size_t a_slot = tc_halo1_a_slot_bytes(planes(h)), b_stage = tc_halo_b_stage_bytes(planes(h), t.n_pad);
-    // fp32-promotion period in (chunk, dx) units of 3 taps: thin layers are latency-bound, give them longer segments
-    int seg = h->seg_chunks > 0 ? h->seg_chunks : (t.n_pad >= 144 ? 1 : (t.n_pad >= 112 ? 2 : 3));
-    seg = std::min(seg, 3 * ((t.cin_pad + 63) / 64));
-    for (; seg >= 1; --seg) {
-      const int na = 2;
-      const long long left = (long long)budget - (long long)na * (long long)a_slot;
-      const int nb = left > 0 ? (int)std::min<long long>(kMaxStages, left / (long long)b_stage) : 0;
-      if (nb >= 3 * seg + 1) {
-        L.halo1 = true;
-        L.halo1_seg = seg;
-        L.halo1_na = na;
-        L.halo1_nb = nb;
-        L.halo1_smem = na * a_slot + nb * b_stage + 1024 + 512 + kRdotSmemBytes;
-        break;
-      }
-    }
-    if (L.halo1) {
-      if (encode_map(h, &L.t1_hi, src_hi, t.cin_pad, src_pitch, n, H, W, kHaloTH + 2, kHalo1W, 64)) return 1;
-      if (planes(h) == 2) {
-        if (encode_map(h, &L.t1_lo, src_lo, t.cin_pad, src_pitch, n, H, W, kHaloTH + 2, kHalo1W, 64)) return 1;
-      } else {
-        L.t1_lo = L.t1_hi;
-      }
-    }
-  }
-
-  // streaming halo kernel: every ring slot is prefetch depth; three (n_pad > 128) or four TMEM accumulation buffers
-  L.halo2 = false;
-  if (pair3x3 && !t.h2_stages.empty()) {
     const size_t a_slot = tc_halo1_a_slot_bytes(planes(h)), b_stage = tc_halo_b_stage_bytes(planes(h), t.n_pad);
     const long long total = 227 * 1024 - (long long)tc_halo2_misc_bytes();
-    const int nst = (int)t.h2_stages.size() / 2;
+    const int nst = 9 * L.p.chunks;
     int na = 2;
     long long nb = (total - na * (long long)a_slot) / (long long)b_stage;
     bool resident = false;
-    static const bool allow_resident = !(getenv("DCSCN_H2_RESIDENT") && atoi(getenv("DCSCN_H2_RESIDENT")) == 0);   // A/B switch
-    if (allow_resident && t.n_tiles == 1 && nst <= kH2MaxStages && (long long)nst * (long long)b_stage + 2 * (long long)a_slot <= total) {
+    if (t.n_tiles == 1 && nst <= kH2MaxStages && (long long)nst * (long long)b_stage + 2 * (long long)a_slot <= total) {
       // thin layers: the whole weight image of this CTA half stays in shared memory, every other byte goes to A boxes
       resident = true;
       nb = nst;
@@ -1147,18 +888,14 @@ static int add_tc_launch(dcscn_handle* h, Plan* pl, const TcLayer& t, const __ha
       L.halo2_na = na;
       L.halo2_nb = (int)nb;
       L.halo2_smem = na * a_slot + (size_t)nb * b_stage + tc_halo2_misc_bytes();
-      L.p.h2_stages = t.d_h2_stages;
       L.p.h2_nstages = nst;
       L.p.h2_nseg = t.h2_nseg;
       L.p.h2_resident = resident ? 1 : 0;
-      L.p.h2_nreg = t.h2_nreg;
-      if (!L.halo1) {   // the A maps of the single-box variants are shared
-        if (encode_map(h, &L.t1_hi, src_hi, t.cin_pad, src_pitch, n, H, W, kHaloTH + 2, kHalo1W, 64)) return 1;
-        if (planes(h) == 2) {
-          if (encode_map(h, &L.t1_lo, src_lo, t.cin_pad, src_pitch, n, H, W, kHaloTH + 2, kHalo1W, 64)) return 1;
-        } else {
-          L.t1_lo = L.t1_hi;
-        }
+      if (encode_map(h, &L.t1_hi, src_hi, t.cin_pad, src_pitch, n, H, W, kHaloTH + 2, kHalo1W)) return 1;
+      if (planes(h) == 2) {
+        if (encode_map(h, &L.t1_lo, src_lo, t.cin_pad, src_pitch, n, H, W, kHaloTH + 2, kHalo1W)) return 1;
+      } else {
+        L.t1_lo = L.t1_hi;
       }
     }
   }
@@ -1274,7 +1011,7 @@ static Plan* get_plan(dcscn_handle* h, int n, int H, int W) {
     pl->fused_index = (int)pl->tc.size() - 1;
     const int parts = rdot_parts(L.p.n_pad, cout);
     pl->fused_last = (klast == 3) && (cout % 16 == 0) && (cout <= 128) && (nch % kColSplit == 0) &&
-                     (((per * 16) % cout == 0) || (parts > 1 && L.halo2 && h->halo == 3 && L.p.n_pad % (per * 16) == 0));
+                     (((per * 16) % cout == 0) || (parts > 1 && L.halo2 && L.p.n_pad % (per * 16) == 0));
     if (pl->fused_last) {
       L.p.epi.rdot_parts = ((per * 16) % cout == 0) ? 1 : parts;
       L.p.epi.mode = EPI_D2S_RDOT;
@@ -1307,31 +1044,6 @@ static Plan* get_plan(dcscn_handle* h, int n, int H, int W) {
 }
 
 // ------------------------------------------------------------------------------------- forward ----
-template <int KC, int NPL>
-static int launch_tc_inst(dcscn_handle* h, const TcLaunch& L, cudaStream_t st) {
-  static bool attr_set_dev[64] = {};   // function attributes are per device
-  bool& attr_set = attr_set_dev[h->cfg.device_id & 63];
-  if (!attr_set) {
-    CUDA_TRY(cudaFuncSetAttribute(conv_tc_kernel<KC, NPL>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-    attr_set = true;
-  }
-  cudaLaunchConfig_t cfg;
-  memset(&cfg, 0, sizeof(cfg));
-  cfg.gridDim = dim3(L.grid);
-  cfg.blockDim = dim3(kTcThreads);
-  cfg.dynamicSmemBytes = L.smem;
-  cfg.stream = st;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = L.p.cluster_size;
-  attr[0].val.clusterDim.y = 1;
-  attr[0].val.clusterDim.z = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = L.p.cluster_size > 1 ? 1 : 0;
-  CUDA_TRY(cudaLaunchKernelEx(&cfg, conv_tc_kernel<KC, NPL>, L.tm_hi, L.tm_lo, L.p, L.stages));
-  return 0;
-}
-
 template <int NPL>
 static int launch_tc_pair(dcscn_handle* h, const TcLaunch& L, cudaStream_t st) {
   static bool attr_set_dev[64] = {};   // function attributes are per device
@@ -1354,68 +1066,9 @@ static int launch_tc_pair(dcscn_handle* h, const TcLaunch& L, cudaStream_t st) {
   cfg.attrs = attr;
   cfg.numAttrs = 1;
   ConvTCParams p = L.p;
-  p.cluster_size = 2;
   p.seg_chunks = L.pair_seg;
   p.pair_stream = L.pair_stream ? 1 : 0;
   CUDA_TRY(cudaLaunchKernelEx(&cfg, conv_tc_pair_kernel<NPL>, L.tm_hi, L.tm_lo, L.tm_w, p, L.pair_stages));
-  return 0;
-}
-
-template <int NPL>
-static int launch_tc_halo(dcscn_handle* h, const TcLaunch& L, cudaStream_t st) {
-  static bool attr_set_dev[64] = {};   // function attributes are per device
-  bool& attr_set = attr_set_dev[h->cfg.device_id & 63];
-  if (!attr_set) {
-    CUDA_TRY(cudaFuncSetAttribute(conv_tc_halo_kernel<NPL>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-    attr_set = true;
-  }
-  cudaLaunchConfig_t cfg;
-  memset(&cfg, 0, sizeof(cfg));
-  cfg.gridDim = dim3(L.halo_grid);
-  cfg.blockDim = dim3(kTcThreads);
-  cfg.dynamicSmemBytes = L.halo_smem;
-  cfg.stream = st;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = 2;
-  attr[0].val.clusterDim.y = 1;
-  attr[0].val.clusterDim.z = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = 1;
-  ConvTCParams p = L.p;
-  p.g = L.hg;
-  p.cluster_size = 2;
-  p.seg_chunks = L.halo_seg;
-  CUDA_TRY(cudaLaunchKernelEx(&cfg, conv_tc_halo_kernel<NPL>, L.th_hi, L.th_lo, L.tm_w, p, L.halo_na, L.halo_nb));
-  return 0;
-}
-
-template <int NPL>
-static int launch_tc_halo1(dcscn_handle* h, const TcLaunch& L, cudaStream_t st) {
-  static bool attr_set_dev[64] = {};   // function attributes are per device
-  bool& attr_set = attr_set_dev[h->cfg.device_id & 63];
-  if (!attr_set) {
-    CUDA_TRY(cudaFuncSetAttribute(conv_tc_halo1_kernel<NPL>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-    attr_set = true;
-  }
-  cudaLaunchConfig_t cfg;
-  memset(&cfg, 0, sizeof(cfg));
-  cfg.gridDim = dim3(L.halo_grid);
-  cfg.blockDim = dim3(kTcThreads);
-  cfg.dynamicSmemBytes = L.halo1_smem;
-  cfg.stream = st;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = 2;
-  attr[0].val.clusterDim.y = 1;
-  attr[0].val.clusterDim.z = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = 1;
-  ConvTCParams p = L.p;
-  p.g = L.hg;
-  p.cluster_size = 2;
-  p.seg_chunks = L.halo1_seg;
-  CUDA_TRY(cudaLaunchKernelEx(&cfg, conv_tc_halo1_kernel<NPL>, L.t1_hi, L.t1_lo, L.tm_w, p, L.halo1_na, L.halo1_nb, h->halo_base));
   return 0;
 }
 
@@ -1474,7 +1127,6 @@ static int launch_tc_halo2(dcscn_handle* h, const TcLaunch& L, cudaStream_t st) 
   cfg.numAttrs = 1;
   ConvTCParams p = L.p;
   p.g = L.hg;
-  p.cluster_size = 2;
   p.seg_chunks = L.halo2_seg;
 #ifdef DCSCN_H2_DEBUG
   {  // diagnostic build: one counter block per launch, dumped by h2_debug_dump() (scripts/r2_h2_timeline.sh)
@@ -1492,9 +1144,7 @@ static int launch_tc_halo2(dcscn_handle* h, const TcLaunch& L, cudaStream_t st) 
     ++g_h2_dbg_launch;
   }
 #endif
-  const bool wide = h->wmap_wide && L.has_wide;
-  CUDA_TRY(cudaLaunchKernelEx(&cfg, conv_tc_halo2_kernel<NPL>, L.t1_hi, L.t1_lo, wide ? L.tm_w_wide : L.tm_w, p, L.halo2_na,
-                              L.halo2_nb, wide ? 1 : 0));
+  CUDA_TRY(cudaLaunchKernelEx(&cfg, conv_tc_halo2_kernel<NPL>, L.t1_hi, L.t1_lo, L.tm_w, p, L.halo2_na, L.halo2_nb));
   return 0;
 }
 
@@ -1516,15 +1166,9 @@ static int launch_tc(dcscn_handle* h, const TcLaunch& Lc, cudaStream_t st) {
     return 0;
   }
   const int npl = planes(h);
-  if (h->pair && h->halo == 3 && L.halo2 && h->kc == 64) return npl == 2 ? launch_tc_halo2<2>(h, L, st) : launch_tc_halo2<1>(h, L, st);
-  if (h->pair && h->halo == 3 && L.p.ksz == 3 && L.pair && h->kc == 64)
-    return fail("internal: 3x3 layer packed for the streaming kernel has no streaming launch shape");
-  if (h->pair && h->halo >= 2 && L.halo1 && h->kc == 64) return npl == 2 ? launch_tc_halo1<2>(h, L, st) : launch_tc_halo1<1>(h, L, st);
-  if (h->pair && h->halo == 1 && L.halo && h->kc == 64) return npl == 2 ? launch_tc_halo<2>(h, L, st) : launch_tc_halo<1>(h, L, st);
-  if (h->pair && L.pair && h->kc == 64) return npl == 2 ? launch_tc_pair<2>(h, L, st) : launch_tc_pair<1>(h, L, st);
-  if (L.p.wpack == nullptr) return fail("internal: single-CTA weight image was not packed for this layer");
-  if (h->kc == 64) return npl == 2 ? launch_tc_inst<64, 2>(h, L, st) : launch_tc_inst<64, 1>(h, L, st);
-  return npl == 2 ? launch_tc_inst<32, 2>(h, L, st) : launch_tc_inst<32, 1>(h, L, st);
+  if (L.halo2) return npl == 2 ? launch_tc_halo2<2>(h, L, st) : launch_tc_halo2<1>(h, L, st);
+  if (L.p.ksz == 3) return fail("internal: 3x3 layer has no streaming launch shape");
+  return npl == 2 ? launch_tc_pair<2>(h, L, st) : launch_tc_pair<1>(h, L, st);
 }
 
 static int mark(dcscn_handle* h, cudaStream_t st) {
@@ -1959,6 +1603,8 @@ int dcscn_create(const dcscn_config* cfg, dcscn_handle** out) {
   cudaDeviceProp prop;
   CUDA_TRY(cudaGetDeviceProperties(&prop, cfg->device_id));
   if (prop.major != 10) return fail("dcscn_create: device %d is sm_%d%d; this library is built for sm_100a (B200) only", cfg->device_id, prop.major, prop.minor);
+  if (prop.multiProcessorCount % 2 != 0)   // the tensor-core kernels run on CTA pairs (two SMs of one TPC)
+    return fail("dcscn_create: device %d has an odd SM count (%d); the CTA-pair tensor-core kernels need an even one", cfg->device_id, prop.multiProcessorCount);
 
   std::unique_ptr<dcscn_handle> h(new dcscn_handle());
   h->cfg = *cfg;
@@ -2298,44 +1944,9 @@ int dcscn_set_option(dcscn_handle* h, const char* key, int64_t value) {
   if (k == "conv_impl") {
     if (value != 0 && value != 1) return fail("conv_impl must be 0 (tcgen05) or 1 (CUDA-core validation)");
     h->conv_impl = (int)value;
-  } else if (k == "kc") {
-    if (value != 64 && value != 32) return fail("kc must be 64 or 32");
-    if (h->kc != (int)value) {
-      h->kc = (int)value;
-      h->cap_px = 0;
-      h->params_dirty = true;  // weight tiles depend on KC
-      h->plans.clear();
-      h->last_plan = nullptr;
-    }
   } else if (k == "ds_impl") {
     if (value != 0 && value != 1) return fail("ds_impl must be 0 (tile kernels) or 1 (first-generation kernels)");
     h->ds_impl = (int)value;
-  } else if (k == "wmap_wide") {
-    h->wmap_wide = value ? 1 : 0;
-  } else if (k == "halo_base") {
-    h->halo_base = (int)value;
-  } else if (k == "halo") {
-    if (value < 0 || value > 3) return fail("halo must be 0, 1, 2 or 3");
-    if ((h->halo == 3) != (value == 3)) {   // the streaming kernel caps column tiles at 160: re-tile and re-pack
-      h->params_dirty = true;
-      h->cap_px = 0;                        // the fused R-CNN1 partial planes may change size
-    }
-    h->plans.clear();
-    h->last_plan = nullptr;
-    h->halo = (int)value;
-  } else if (k == "pair") {
-    if (h->pair != (value ? 1 : 0)) {
-      h->pair = value ? 1 : 0;
-      h->cap_px = 0;
-      h->params_dirty = true;   // the two kernels use different packed weight layouts
-      h->plans.clear();
-      h->last_plan = nullptr;
-    }
-  } else if (k == "cluster") {
-    if (value != 1 && value != 2 && value != 4) return fail("cluster must be 1, 2 or 4");
-    h->cluster = (int)value;
-    h->plans.clear();
-    h->last_plan = nullptr;
   } else if (k == "fuse_last") {
     h->fuse_last = value ? 1 : 0;
   } else if (k == "timing") {
@@ -2345,8 +1956,6 @@ int dcscn_set_option(dcscn_handle* h, const char* key, int64_t value) {
     h->wgrad_impl = (int)value;
   } else if (k == "l1_loss") {
     h->l1_loss = value ? 1 : 0;
-  } else if (k == "wgrad_halo") {
-    h->wgrad_halo = value ? 1 : 0;
   } else if (k == "wgrad_taps") {
     if (value < 0 || value > 3) return fail("wgrad_taps must be 0 (automatic) .. 3");
     h->wgrad_taps = (int)value;

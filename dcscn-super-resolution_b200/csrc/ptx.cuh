@@ -90,25 +90,6 @@ __device__ __forceinline__ void tma_load_4d(void* smem_dst, const CUtensorMap* t
       : "memory");
 }
 
-// 1-D bulk copy global -> shared (16-byte aligned, size multiple of 16).
-__device__ __forceinline__ void bulk_load(void* smem_dst, const void* gsrc, uint32_t bytes, uint64_t* bar) {
-  asm volatile(
-      "cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
-          smem_u32(smem_dst)),
-      "l"(reinterpret_cast<uint64_t>(gsrc)), "r"(bytes), "r"(smem_u32(bar))
-      : "memory");
-}
-
-// Same, delivered to the same shared-memory offset (and mbarrier offset) of every CTA in `cta_mask`.
-__device__ __forceinline__ void bulk_load_multicast(void* smem_dst, const void* gsrc, uint32_t bytes, uint64_t* bar,
-                                                    uint16_t cta_mask) {
-  asm volatile(
-      "cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster [%0], [%1], %2, [%3], %4;" ::
-          "r"(smem_u32(smem_dst)),
-      "l"(reinterpret_cast<uint64_t>(gsrc)), "r"(bytes), "r"(smem_u32(bar)), "h"(cta_mask)
-      : "memory");
-}
-
 // ----------------------------------------------------------------- tcgen05 ----
 __device__ __forceinline__ void tmem_alloc(uint32_t* smem_result, uint32_t cols) {
   asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(smem_result)),
@@ -145,15 +126,6 @@ __device__ __forceinline__ void mma_f16_ss(uint32_t tmem_d, uint64_t desc_a, uin
 __device__ __forceinline__ void mma_commit(uint64_t* bar) {
   asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar))
                : "memory");
-}
-
-// Same arrival on the barrier at this offset in every CTA of `cta_mask`.
-__device__ __forceinline__ void mma_commit_multicast(uint64_t* bar, uint16_t cta_mask) {
-  asm volatile(
-      "tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(
-          smem_u32(bar)),
-      "h"(cta_mask)
-      : "memory");
 }
 
 // TMEM -> registers: this warp's 32 lanes x 16 consecutive fp32 columns.

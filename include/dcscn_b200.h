@@ -55,7 +55,8 @@ typedef struct dcscn_config {
   int32_t precision;              /* DCSCN_PRECISION_* */
 } dcscn_config;
 
-/* SuperResolution(flags) + build_graph() + init_session (DCSCN.py:29, :222; tf_graph.py:65). */
+/* SuperResolution(flags) + build_graph() + init_session (DCSCN.py:29, :222; tf_graph.py:65).  Fails on a device that is
+ * not sm_100a or has an odd SM count (the tensor-core kernels run on CTA pairs). */
 int dcscn_create(const dcscn_config* cfg, dcscn_handle** out);
 /* sess.close() */
 int dcscn_destroy(dcscn_handle* h);
@@ -165,13 +166,7 @@ int dcscn_dropout_mask(dcscn_handle* h, const char* tensor, uint32_t seed, int n
 int dcscn_get_activation(dcscn_handle* h, const char* tensor, float* host_data, int64_t numel);
 
 /* Options: "conv_impl" 0 = tcgen05 (default), 1 = CUDA-core fp32 validation kernels;
- *          "kc" 64 | 32 = K-chunk (channels per pipeline stage) of the tensor-core kernel;
  *          "seg_chunks" = pipeline stages per fp32-promotion segment (default 0 = automatic: 2, or 3 for thin layers);
- *          "halo" 0 | 1 | 2 | 3 = 3x3 layers: one A tile per tap (0), three 18x8 boxes per channel chunk (1), one
- *                     18x10 box per channel chunk serving all nine taps with two-pass segments (2), or the same box with
- *                     streaming weight stages and split correction / dominant accumulators (3, default);
- *          "pair" 1 | 0 = CTA-pair kernel (tcgen05 cta_group::2, weight tiles split across two SMs; default 1);
- *          "cluster" 1 | 2 | 4 = CTAs per cluster multicasting weight tiles in the single-CTA kernel (default 1);
  *          "fuse_last" 1 | 0 = compute the per-pixel half of R-CNN1 inside the last Up-PS epilogue (default 1);
  *          "timing" 0 | 1 = record per-launch CUDA events (see dcscn_get_timings);
  *          "store_mode" 2 | 0 | 1 = fp16 plane stores of the tensor-core epilogues: 32-byte stores with neighbouring lanes

@@ -79,7 +79,7 @@ if "B" in which:
         if prelu:
             w0["%s/prelu/%s_prelu" % (scope, base)] = np.full(cout, 0.1, np.float32)
     order = np.random.RandomState(1).permutation(ds.count)
-    for opts in [{}, {"host": 1}, {"wgrad_impl": 1}, {"host_repack": 1}, {"halo": 2}, {"conv_impl": 1}]:
+    for opts in [{}, {"host": 1}, {"wgrad_impl": 1}, {"host_repack": 1}, {"conv_impl": 1}]:
         eng = E.Engine(E.make_config(dropout_keep=0.8, **KW))
         eng.set_params(w0)
         host = opts.pop("host", 0) if "host" in opts else 0

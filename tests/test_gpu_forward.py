@@ -74,9 +74,7 @@ def small():
     eng.close()
 
 
-@pytest.mark.parametrize("n,h,w", [(1, 20, 37), (2, 48, 48), (1, 1, 1), (1, 3, 130), (3, 17, 9), (1, 129, 2)])
-def test_small_graph_every_layer(small, n, h, w):
-    cfg, wts, eng = small
+def check_every_layer(cfg, wts, eng, n, h, w):
     g = np.random.RandomState(n * 1000 + h * 10 + w)
     x = (g.rand(n, h, w, 1) * 255).astype(np.float32)
     x2 = (g.rand(n, 2 * h, 2 * w, 1) * 255).astype(np.float32)
@@ -91,6 +89,28 @@ def test_small_graph_every_layer(small, n, h, w):
         a = eng.get_activation(name, ref.shape)
         # fp32-level agreement relative to the layer's dynamic range
         assert np.abs(a - ref).max() <= 4e-6 * max(1.0, np.abs(ref).max()) + 1e-4, name
+
+
+@pytest.mark.parametrize("n,h,w", [(1, 20, 37), (2, 48, 48), (1, 1, 1), (1, 3, 130), (3, 17, 9), (1, 129, 2)])
+def test_small_graph_every_layer(small, n, h, w):
+    check_every_layer(*small, n, h, w)
+
+
+@pytest.fixture(scope="module", params=[5, 1], ids=["cnn5", "cnn1"])
+def small_other_ksz(request):
+    kw = dict(SMALL, cnn_size=request.param)
+    cfg = O.OracleConfig(**kw)
+    w = O.he_init_weights(cfg, seed=0)
+    eng = make_engine(kw, w)
+    yield cfg, w, eng
+    eng.close()
+
+
+@pytest.mark.parametrize("n,h,w", [(1, 20, 37), (3, 17, 9), (1, 3, 130)])
+def test_small_graph_other_kernel_sizes(small_other_ksz, n, h, w):
+    """conv_tc_pair_kernel's two-pass mode with more than one tap: every 5x5 layer runs on it, and so does a 1x1 layer
+    wider than 128 columns (here Up-PS at cnn_size 1).  B2 stays 3x3, so the streaming kernel runs in the same forward."""
+    check_every_layer(*small_other_ksz, n, h, w)
 
 
 def test_validation_kernels_agree_with_tensor_core_path(small):
@@ -111,42 +131,6 @@ def test_validation_kernels_agree_with_tensor_core_path(small):
     y_strict = gpu_forward(eng, x, x2)
     eng.set_option("seg_chunks", 0)
     assert np.abs(y_strict - y64).max() <= 1.5 * max(err_ref, 5e-4), (float(np.abs(y_strict - y64).max()), err_ref)
-
-
-@pytest.mark.parametrize("opts", [{"halo": 2}, {"halo": 1}, {"halo": 0}, {"pair": 0}, {"pair": 0, "cluster": 2}, {"pair": 0, "cluster": 4}],
-                         ids=["halo1-single-box", "halo-three-box", "pair-two-pass", "single-cta", "multicast-2", "multicast-4"])
-def test_earlier_kernel_generations_stay_correct(small, opts):
-    """The selectable predecessors of the streaming kernel (A/B baselines for the profiles under profiles/): every one
-    has to keep producing the same forward within the stress bound, or be deleted."""
-    cfg, wts, eng = small
-    g = np.random.RandomState(21)
-    x = (g.rand(2, 26, 35, 1) * 255).astype(np.float32)
-    x2 = (g.rand(2, 52, 70, 1) * 255).astype(np.float32)
-    y64 = O.Oracle(cfg, wts, torch.float64).forward(x.astype(np.float64), x2.astype(np.float64))
-    y32 = O.Oracle(cfg, wts, torch.float32).forward(x, x2)
-    defaults = {"halo": 3, "pair": 1, "cluster": 1}
-    try:
-        for k, v in opts.items():
-            eng.set_option(k, v)
-        y = gpu_forward(eng, x, x2)
-    finally:
-        for k in opts:
-            eng.set_option(k, defaults[k])
-    assert np.isfinite(y).all()
-    assert np.abs(y - y64).max() <= max(TOL_DEFAULT_STRESS, stress_bound(y32, y64))
-
-
-def test_kc32_pipeline_variant(small):
-    cfg, wts, eng = small
-    g = np.random.RandomState(8)
-    x = (g.rand(1, 40, 24, 1) * 255).astype(np.float32)
-    x2 = (g.rand(1, 80, 48, 1) * 255).astype(np.float32)
-    y64 = O.Oracle(cfg, wts, torch.float64).forward(x.astype(np.float64), x2.astype(np.float64))
-    y32 = O.Oracle(cfg, wts, torch.float32).forward(x, x2)
-    eng.set_option("kc", 32)
-    y = gpu_forward(eng, x, x2)
-    eng.set_option("kc", 64)
-    assert np.abs(y - y64).max() <= stress_bound(y32, y64)
 
 
 def test_forward_host_matches_device_call_and_plan_cache(small):
@@ -280,6 +264,9 @@ def test_errors_are_loud():
         eng.set_param("CNN1/conv_B", np.zeros(3, np.float32))  # wrong size
     with pytest.raises(E.EngineError):
         eng.set_option("conv_impl", 7)
+    for key in ("halo", "halo_base", "pair", "cluster", "kc", "wmap_wide", "wgrad_halo"):   # removed kernel selectors
+        with pytest.raises(E.EngineError):
+            eng.set_option(key, 1)
     eng.close()
 
 
